@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the nnaudio-b200 hot path (contract: task brief §④ / base contract).
 
-  python bench.py --gpus N --steps K --warmup W [--workload cfg2] [--impl reference]
+  python bench.py --gpus N --steps K --warmup W [--workload cfg2] [--impl reference] [--dump-outputs DIR]
 
 A *step* is one pass of the hot path over one batch of synthetic white noise:
 by default ``cfg2`` of BASELINE.json (MelSpectrogram n_fft=2048 hop=512
@@ -15,6 +15,10 @@ region).  Under torchrun (N > 1) every rank processes its own batch shard
 ``--impl reference`` times the CPU arm instead: the NumPy oracle port of the
 reference's conv1d path (oracle/nnaudio_oracle.py) on the host cores — the
 reference itself is Python and cannot travel to the GPU box.
+
+``--dump-outputs DIR`` writes the spectrograms the last timed step of the headline workload returned as
+``DIR/<workload>.npy`` (float32; a seeded sample of whole clips when they exceed 64 MB).  The inputs are
+seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -27,6 +31,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True  # the tree may be read-only: no __pycache__ from the modules imported here
 
 # torchrun exports OMP_NUM_THREADS=1 to its workers.  The CPU arm is meant to use the host cores
 # ("all the host threads it can use"), and BLAS sizes its pool when it is first loaded, so put the
@@ -232,7 +237,7 @@ def static_traffic(workload):
         return None
 
 
-REF_DIR = os.path.join(ROOT, "baseline", "_ref")
+REF_DIR = os.path.join(ROOT, "oracle", "_ref")
 
 
 def reference_available():
@@ -240,8 +245,8 @@ def reference_available():
 
 
 def _reference_module(workload):
-    """The UNMODIFIED reference module of a workload, imported from baseline/_ref
-    (baseline/install_ref.sh; pip --target install of /root/reference/Installation)."""
+    """The UNMODIFIED reference module of a workload, imported from oracle/_ref
+    (copied there by oracle/install_ref.sh during build())."""
     if REF_DIR not in sys.path:
         sys.path.insert(0, REF_DIR)
     import importlib
@@ -297,7 +302,7 @@ def reference_cpu_arm(workload, steps, warmup, budget_s):
     return {
         "value": clips * T * steps / dt, "unit": "frames/s", "cores": threads, "kind": "reference",
         "sample": f"{clips} clip(s) x {w['L']} samples of {workload} per step, {steps} steps, unmodified "
-                  f"nnAudio 0.3.3 {w['cls']} (baseline/_ref) on CPU, torch {torch.__version__} conv1d, "
+                  f"nnAudio 0.3.3 {w['cls']} (oracle/_ref) on CPU, torch {torch.__version__} conv1d, "
                   f"{threads} threads (fastest of all / 2 / 4 / 8 of {avail} cores), {dt:.1f}s",
         "ms_per_step": 1e3 * dt / steps,
     }
@@ -351,6 +356,23 @@ def reference_gpu_leg(workload, dev, budget_s=20.0):
     return {"value": None, "unavailable": last_err}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, name, y):
+    """``out_dir/<name>.npy``: ``y`` (a CPU tensor, clips first) as float32, or, above DUMP_LIMIT_BYTES, the
+    clips of a fixed seeded sample in ascending order."""
+    import numpy as np
+
+    a = y.float().numpy()
+    per_clip = a[0].nbytes
+    if a.nbytes > DUMP_LIMIT_BYTES:
+        keep = max(1, DUMP_LIMIT_BYTES // per_clip)
+        a = a[np.sort(np.random.RandomState(0).choice(a.shape[0], keep, replace=False))]
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, f"{name}.npy"), np.ascontiguousarray(a))
+
+
 # ----------------------------------------------------------------------------
 def main():
     # stdout carries exactly ONE line (the JSON); libraries that print there (NCCL's version
@@ -379,7 +401,8 @@ def _run():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--e2e-chunks", type=int, default=8)
     ap.add_argument("--no-workloads", action="store_true", help="skip the secondary configs (stft2048, cfg3, cfg4, cfg5)")
-    ap.add_argument("--workload-steps", type=int, default=10)
+    ap.add_argument("--workload-steps", type=int, default=None,
+                    help="timed steps of each secondary config (default: --steps)")
     ap.add_argument("--no-reference-gpu", action="store_true", help="skip the reference's cuDNN leg")
     ap.add_argument("--no-numa-bind", action="store_true")
     ap.add_argument("--watchdog", type=int, default=900, help="seconds after which a stuck run is aborted")
@@ -394,7 +417,11 @@ def _run():
                     help="SMs kept free for the concurrent NCCL gather (default: by world size)")
     ap.add_argument("--nccl-max-ctas", type=int, default=-1,
                     help="-1 = same as the SM reserve (default), 0 = NCCL's own default")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the headline workload's output of the last timed step to DIR/<workload>.npy")
     args = ap.parse_args()
+    if args.workload_steps is None:
+        args.workload_steps = args.steps
     if args.warmup < 3:
         args.warmup = 3
 
@@ -418,10 +445,10 @@ def _run():
             return None
         if reference_available():
             res = reference_cpu_arm(args.workload, args.steps, args.warmup, budget_s=120.0)
-            arm = "the UNMODIFIED reference (baseline/_ref, nnAudio 0.3.3) on the host cores: torch conv1d (oneDNN)"
+            arm = "the UNMODIFIED reference (oracle/_ref, nnAudio 0.3.3) on the host cores: torch conv1d (oneDNN)"
         else:
             res = cpu_arm(args.workload, args.steps, args.warmup, budget_s=120.0)
-            arm = "CPU oracle port of the reference conv1d path (baseline/_ref not installed)"
+            arm = "CPU oracle port of the reference conv1d path (oracle/_ref not installed)"
         line = {
             "impl": "reference", "metric": metric, "value": res["value"], "unit": "frames/s",
             "n_gpus": args.gpus, "steps": args.steps, "warmup": args.warmup,
@@ -526,7 +553,7 @@ def _run():
     if gather_impl in ("symm", "peer") and args.reserve_sms is None:
         reserve = 0  # the copy engines do the gather: the kernels keep every SM
 
-    def measure(name, steps, warmup, gather):
+    def measure(name, steps, warmup, gather, keep_output=False):
         """One workload, inputs resident in HBM: ``steps`` timed steps between two CUDA events on the
         launching stream (max over ranks), the framed contraction timed per launch with in-stream
         events (nnab_profile_*), clocks sampled through NVML during the timed region."""
@@ -589,10 +616,11 @@ def _run():
             sampler.start()
             sync_all()
             e0.record()
-            run_steps(steps)
+            y = run_steps(steps)
             e1.record()
             sync_all()
             clocks = sampler.stop()
+            y = y.cpu() if keep_output else None
             _C.profile_enable(False)
             launches = _C.launch_count() - launches0
             framed_ms, framed_n = _C.profile_read()
@@ -640,13 +668,17 @@ def _run():
             "l2": f"{n_rot} rotating input batch(es) of {batch_bytes / 1e6:.0f} MB (> 126 MB L2 in total), no flush",
             "dtype": "bf16x3 split (fp32-equivalent), f32 accumulate" if used_tc else "f32",
         }
-        return res, mod, out_shape, w
+        return res, mod, out_shape, w, y
 
-    main, mod, out_shape, w = measure(args.workload, args.steps, args.warmup, gather=True)
+    main, mod, out_shape, w, y_last = measure(args.workload, args.steps, args.warmup, gather=True,
+                                              keep_output=bool(args.dump_outputs) and rank == 0)
+    if y_last is not None:
+        dump_outputs(args.dump_outputs, args.workload, y_last)
+    del y_last
     B = w["B"]
     no_gather = None
     if world > 1:  # SURVEY.md 8(e): frames/s with and without the gather
-        ng, m_ng, _, _ = measure(args.workload, args.steps, args.warmup, gather=False)
+        ng, m_ng, _, _, _ = measure(args.workload, args.steps, args.warmup, gather=False)
         del m_ng
         no_gather = {"value": ng["value"], "ms_per_step": ng["ms_per_step"],
                      "what": "same run, transform only (shards stay on their GPUs)"}
@@ -714,7 +746,7 @@ def _run():
             for i in range(3):
                 pipe(x_hosts[i & 1], y_host, device=dev)
             sync_all()
-            n_e2e = max(args.steps, 20)
+            n_e2e = args.steps
             a, b_ = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             a.record()
             for i in range(n_e2e):
@@ -747,7 +779,7 @@ def _run():
         torch.cuda.empty_cache()
         for name in [n for n in SECONDARY if n != args.workload]:
             try:
-                res, m2, _, _ = measure(name, steps=args.workload_steps, warmup=3, gather=False)
+                res, m2, _, _, _ = measure(name, steps=args.workload_steps, warmup=3, gather=False)
                 del m2
                 others[name] = res
             except Exception as e:  # noqa: BLE001  (never cost the headline line)

@@ -3,12 +3,59 @@ build container) and the test-suite (runs the oracle and the CUDA path).
 
 Inputs are regenerated from the spec (NumPy ``RandomState`` / ``scipy.signal.chirp``
 are platform-stable), so only the reference OUTPUTS are stored in
-``ref_outputs.npz``.
+``ref_outputs.npz``, and of each output only a fixed sample of its entries
+(``sample_index``) plus its extreme entries, so that the stored files stay small.
 """
 from __future__ import annotations
 
+import zlib
+
 import numpy as np
 from scipy.signal import chirp
+
+GOLDEN_SAMPLES = 2048  # entries kept of each stored reference array
+
+
+def sample_index(key: str, shape, peaks=()) -> np.ndarray:
+    """Sorted flat (C-order) indices of the entries of the reference array ``key`` that are stored: all
+    of them for a small array, else ``GOLDEN_SAMPLES`` drawn with a seed derived from ``key``, plus
+    ``peaks`` (the array's extremes, stored beside the values so that max-normalised errors use the full
+    array's maximum)."""
+    n = int(np.prod(shape))
+    if n <= GOLDEN_SAMPLES:
+        return np.arange(n)
+    idx = np.random.RandomState(zlib.crc32(key.encode())).choice(n, GOLDEN_SAMPLES, replace=False)
+    return np.union1d(idx, np.asarray(peaks, dtype=np.int64))
+
+
+def array_peaks(a: np.ndarray) -> np.ndarray:
+    """Flat indices of max |a|, max a and min a."""
+    a = np.asarray(a).reshape(-1)
+    return np.array([np.abs(a).argmax(), a.argmax(), a.argmin()], dtype=np.int64)
+
+
+def pack_sampled(outputs: dict) -> dict:
+    """{key: full array} -> the arrays of a sampled fixture file (values, shape and peaks per key)."""
+    packed = {}
+    for key, a in outputs.items():
+        peaks = array_peaks(a)
+        packed[key] = np.asarray(a, dtype=np.float32).reshape(-1)[sample_index(key, a.shape, peaks)]
+        packed[key + "|shape"] = np.array(a.shape, dtype=np.int64)
+        packed[key + "|peaks"] = peaks
+    return packed
+
+
+def istft_spectrogram(case, wsin=None, wcos=None) -> np.ndarray:
+    """Spectrogram input of an ISTFT case: seeded noise ('module'), or the fp64 oracle STFT (rounded to
+    fp32) of seeded noise with the bases ``wsin`` / ``wcos`` of the case's STFT module ('roundtrip')."""
+    cid, n_fft, hop, win, kind, spec = case
+    rng = np.random.RandomState(spec["seed"])
+    if kind == "module":
+        return rng.standard_normal(spec["shape"]).astype(np.float32)
+    from nnaudio_oracle import stft
+
+    x = rng.standard_normal(spec["shape"]).astype(np.float32)
+    return stft(x, wsin, wcos, hop, center=True, pad_mode="reflect", output_format="Complex").astype(np.float32)
 
 
 def make_input(spec) -> np.ndarray:
@@ -129,7 +176,8 @@ SWEEP_CTOR = dict(sr=44100, fmin=55, n_bins=207, bins_per_octave=24)
 
 
 # Inverse STFT cases (SURVEY.md §8f next #2): id, n_fft, hop, window, kind, spec
-#   'roundtrip': X = reference STFT(iSTFT=True)(x), y = .inverse(X, onesided=True, length=L|None)
+#   'roundtrip': X = STFT of x (istft_spectrogram), y = reference STFT(iSTFT=True).inverse(X, onesided=True,
+#                length=L|None)
 #   'module'   : y = reference iSTFT(...)(X_random, onesided=False)
 ISTFT_CASES = [
     ("istft_roundtrip_512", 512, 128, "hann", "roundtrip", dict(seed=70, shape=(2, 4000), length=4000)),

@@ -9,6 +9,8 @@ outputs are committed:
                          Installation/tests/ground-truths/*.npy (test fixtures,
                          not source code) — pinned by tests/test_cqt.py:94-262
 
+Both .npz files keep a seeded sample of each array's entries (cases.pack_sampled).
+
 (The Combined_Frequency_Periodicity / CFP fixtures have their own generator, make_golden_cfp.py ->
 ref_cfp.npz / ref_cfp.json.)
 
@@ -30,9 +32,11 @@ REF = os.environ.get("NNAUDIO_REF", "/root/reference/Installation")
 sys.dont_write_bytecode = True
 sys.path.insert(0, REF)
 sys.path.insert(0, HERE)
+sys.path.insert(0, os.path.join(HERE, "..", "..", "oracle"))
 
 from cases import (CASES, DESIGN_CASES, ERROR_CASES, GRAD_CASES, SWEEP_FORWARD, sweep_input, ISTFT_CASES, ISTFT_GRAD_CASES, REF_GROUND_TRUTHS,  # noqa: E402
-                   SWEEP_CTOR, WGRAD_CASES, attribute_surface, loss_weights, make_input, out_key)
+                   SWEEP_CTOR, WGRAD_CASES, attribute_surface, istft_spectrogram, loss_weights, make_input,
+                   out_key, pack_sampled)
 
 from nnAudio import features as ref_features  # noqa: E402
 
@@ -126,45 +130,40 @@ def main():
         print(f"{cid:60s} -> {errors[cid]}")
     with open(os.path.join(HERE, "ref_errors.json"), "w") as f:
         json.dump(errors, f, indent=1, sort_keys=True)
-    # inverse STFT: spectrogram inputs AND waveform outputs of the reference
-    for cid, n_fft, hop, win, kind, spec in ISTFT_CASES:
-        rng = np.random.RandomState(spec["seed"])
+    # inverse STFT: waveform outputs of the reference (the spectrogram inputs are regenerated by the tests)
+    for case in ISTFT_CASES:
+        cid, n_fft, hop, win, kind, spec = case
         with warnings.catch_warnings():
             warnings.simplefilter("ignore")
             if kind == "roundtrip":
                 st = ref_features.STFT(n_fft=n_fft, hop_length=hop, window=win, iSTFT=True, verbose=False)
-                x = torch.from_numpy(rng.standard_normal(spec["shape"]).astype(np.float32))
+                X = torch.from_numpy(istft_spectrogram(case, st.wsin.numpy(), st.wcos.numpy()))
                 with torch.no_grad():
-                    X = st(x)
                     y = st.inverse(X, onesided=True, length=spec["length"])
             else:
                 im = ref_features.iSTFT(n_fft=n_fft, hop_length=hop, window=win, verbose=False)
-                X = torch.from_numpy(rng.standard_normal(spec["shape"]).astype(np.float32))
+                X = torch.from_numpy(istft_spectrogram(case))
                 with torch.no_grad():
                     y = im(X, onesided=False)
-        outputs[cid + "|X"] = X.numpy().astype(np.float32)
         outputs[cid + "|y"] = y.numpy().astype(np.float32)
         print(f"{cid:60s} X{tuple(X.shape)} -> y{tuple(y.shape)}")
     # gradient of the inverse STFT w.r.t. its spectrogram input
-    for cid, n_fft, hop, win, kind, spec in ISTFT_GRAD_CASES:
-        rng = np.random.RandomState(spec["seed"])
+    for case in ISTFT_GRAD_CASES:
+        cid, n_fft, hop, win, kind, spec = case
         with warnings.catch_warnings():
             warnings.simplefilter("ignore")
             if kind == "roundtrip":
                 st = ref_features.STFT(n_fft=n_fft, hop_length=hop, window=win, iSTFT=True, verbose=False)
-                x = torch.from_numpy(rng.standard_normal(spec["shape"]).astype(np.float32))
-                with torch.no_grad():
-                    X = st(x)
-                X = X.clone().requires_grad_(True)
+                X = torch.from_numpy(istft_spectrogram(case, st.wsin.numpy(), st.wcos.numpy()))
+                X.requires_grad_(True)
                 y = st.inverse(X, onesided=True, length=spec["length"])
             else:
                 im = ref_features.iSTFT(n_fft=n_fft, hop_length=hop, window=win, verbose=False)
-                X = torch.from_numpy(rng.standard_normal(spec["shape"]).astype(np.float32))
+                X = torch.from_numpy(istft_spectrogram(case))
                 X.requires_grad_(True)
                 y = im(X, onesided=False)
         w = torch.from_numpy(loss_weights(cid, tuple(y.shape)))
         (y * w).sum().backward()
-        outputs[cid + "|X"] = X.detach().numpy().astype(np.float32)
         outputs[cid + "|dX"] = X.grad.numpy().astype(np.float32)
         print(f"{cid:60s} X{tuple(X.shape)} y{tuple(y.shape)} -> dX{tuple(X.grad.shape)}")
     # input gradients through the reference's own autograd path
@@ -191,7 +190,7 @@ def main():
         for n in names:
             outputs[f"wgrad|{cid}|{n}"] = params[n].grad.numpy().astype(np.float32)
             print(f"{'wgrad|' + cid + '|' + n:60s} {tuple(params[n].grad.shape)}")
-    np.savez_compressed(os.path.join(HERE, "ref_outputs.npz"), **outputs)
+    np.savez_compressed(os.path.join(HERE, "ref_outputs.npz"), **pack_sampled(outputs))
     with open(os.path.join(HERE, "ref_buffers.json"), "w") as f:
         json.dump(buffers, f, indent=1, sort_keys=True)
 
@@ -213,7 +212,7 @@ def main():
         ok = np.allclose(y.numpy(), gt, rtol=1e-3, atol=1e-3)
         print(f"{key:40s} gt{gt.shape} ref reproduces: {ok}  maxabs {np.abs(y.numpy()-gt).max():.3e}")
         assert ok, key
-    np.savez_compressed(os.path.join(HERE, "ref_ground_truths.npz"), **gts)
+    np.savez_compressed(os.path.join(HERE, "ref_ground_truths.npz"), **pack_sampled(gts))
     print("wrote fixtures to", HERE)
 
 

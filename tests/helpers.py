@@ -19,7 +19,8 @@ for p in (ROOT, GOLDEN, os.path.join(ROOT, "oracle")):
         sys.path.insert(0, p)
 
 import nnaudio_oracle as oracle  # noqa: E402  (test infrastructure only)
-from cases import CASES, REF_GROUND_TRUTHS, SWEEP_CTOR, make_input, out_key  # noqa: E402,F401
+from cases import (CASES, REF_GROUND_TRUTHS, SWEEP_CTOR, istft_spectrogram, make_input,  # noqa: E402,F401
+                   out_key, sample_index)
 
 import nnaudio_b200 as nb  # noqa: E402
 
@@ -28,18 +29,54 @@ _REF_GT = None
 _REF_BUF = None
 
 
+class Sampled:
+    """A stored reference array: its full ``shape`` and its ``values`` at the flat indices ``idx``
+    (tests/golden/cases.py: ``sample_index``; they include the entries of max |a|, max a and min a).
+    Compare a full-size result with ``pick(result)`` against ``values``."""
+
+    def __init__(self, key, shape, peaks, values):
+        self.shape = tuple(int(s) for s in shape)
+        self.idx = sample_index(key, self.shape, peaks)
+        self.values = values
+        assert values.shape == self.idx.shape, key
+
+    def pick(self, a):
+        """The stored entries of ``a``: an array of the full size (unit axes may differ), or a mask whose
+        shape lacks the trailing (real, imag) axis of a complex-format output."""
+        a = np.asarray(a)
+        if a.shape != self.shape and a.shape + (2,) == self.shape:
+            a = np.broadcast_to(a[..., None], self.shape)
+        assert a.size == int(np.prod(self.shape)), (a.shape, self.shape)
+        return a.reshape(-1)[self.idx]
+
+
+def _load_sampled(name):
+    d = np.load(os.path.join(GOLDEN, name))
+    return {k: Sampled(k, d[k + "|shape"], d[k + "|peaks"], d[k])
+            for k in d.files if not k.endswith(("|shape", "|peaks"))}
+
+
 def ref_outputs():
     global _REF_OUT
     if _REF_OUT is None:
-        _REF_OUT = dict(np.load(os.path.join(GOLDEN, "ref_outputs.npz")))
+        _REF_OUT = _load_sampled("ref_outputs.npz")
     return _REF_OUT
 
 
 def ref_ground_truths():
     global _REF_GT
     if _REF_GT is None:
-        _REF_GT = dict(np.load(os.path.join(GOLDEN, "ref_ground_truths.npz")))
+        _REF_GT = _load_sampled("ref_ground_truths.npz")
     return _REF_GT
+
+
+def istft_input(case):
+    """The spectrogram the reference inverted for an ISTFT case (cases.ISTFT_CASES / ISTFT_GRAD_CASES)."""
+    cid, n_fft, hop, win, kind, spec = case
+    if kind == "module":
+        return istft_spectrogram(case)
+    st = build("STFT", dict(n_fft=n_fft, hop_length=hop, window=win, iSTFT=True))
+    return istft_spectrogram(case, st.wsin.detach().cpu().numpy(), st.wcos.detach().cpu().numpy())
 
 
 def ref_buffers():

@@ -25,9 +25,9 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert d["value"] > 0 and d["n_gpus"] == 1 and d["data"] == "synthetic"
     assert d["config"]["workload"].startswith("cfg2")
     cb = d["cpu_baseline"]
-    # "reference" when baseline/_ref (the unmodified reference, baseline/install_ref.sh) is installed,
+    # "reference" when oracle/_ref (the unmodified reference, oracle/install_ref.sh) is installed,
     # else the NumPy oracle port
-    want = "reference" if os.path.isdir(os.path.join(ROOT, "baseline", "_ref", "nnAudio")) else "port"
+    want = "reference" if os.path.isdir(os.path.join(ROOT, "oracle", "_ref", "nnAudio")) else "port"
     assert cb["kind"] == want and cb["value"] == d["value"] and cb["cores"] >= 1 and cb["sample"]
     e2e = d["e2e"]
     assert e2e["value"] == d["value"] and e2e["h2d_bytes_per_step"] == 0 and e2e["d2h_bytes_per_step"] == 0

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """CFP timing on one B200 (not part of bench.py's line): our dense-contraction formulation
-(nnaudio_b200.features.CFP) and, when baseline/_ref is present, the unmodified reference module on the same
+(nnaudio_b200.features.CFP) and, when oracle/_ref is present, the unmodified reference module on the same
 GPU (torch.stft + torch.fft through cuFFT), same input, CUDA events after warm-up.
 
     python tools/bench_cfp.py [--batch 16] [--seconds 10] [--steps 10]
@@ -48,7 +48,7 @@ def main():
     frames = args.batch * y.shape[-1]
     out = {"workload": f"CFP default (fr=2, fs=16000, hop=320), {args.batch} x {args.seconds:g} s", "frames": frames,
            "ours_ms": ms, "ours_frames_per_s": frames / ms * 1e3}
-    ref_dir = os.path.join(ROOT, "baseline", "_ref")
+    ref_dir = os.path.join(ROOT, "oracle", "_ref")
     if os.path.isdir(os.path.join(ref_dir, "nnAudio")):
         import scipy.signal
         import scipy.signal.windows

@@ -2,7 +2,7 @@
 """Gammatonegram timing on one B200 (cfg2 shape: 64 x 10 s @ 22.05 kHz, n_fft 2048, hop 512, 64 bins):
 dense bank on the tensor cores (NNAB_FB_PLANES=1: operand planes + second tcgen05 contraction), the
 round-1 path (NNAB_FB_PLANES=0: fp32 power spectrogram + CUDA-core GEMM), the STFT power alone for scale,
-and the unmodified reference on the same GPU when baseline/_ref is present.  CUDA events after warm-up.
+and the unmodified reference on the same GPU when oracle/_ref is present.  CUDA events after warm-up.
 """
 import json
 import os
@@ -52,7 +52,7 @@ def main():
         out["stft_magnitude_ms"] = timed(lambda: stft(nxt()))
     out["frames"] = frames
     out["planes_frames_per_s"] = frames / out["planes_ms"] * 1e3
-    ref_dir = os.path.join(ROOT, "baseline", "_ref")
+    ref_dir = os.path.join(ROOT, "oracle", "_ref")
     if os.path.isdir(os.path.join(ref_dir, "nnAudio")):
         sys.path.insert(0, ref_dir)
         from nnAudio.features.gammatone import Gammatonegram as Ref

@@ -49,7 +49,7 @@ def main():
     import nnaudio_b200 as nb
 
     ref_features = None
-    ref_dir = os.path.join(ROOT, "baseline", "_ref")
+    ref_dir = os.path.join(ROOT, "oracle", "_ref")
     if os.path.isdir(os.path.join(ref_dir, "nnAudio")):
         sys.path.insert(0, ref_dir)
         from nnAudio import features as ref_features
