@@ -23,7 +23,11 @@ Same class names, constructor arguments (names, order, defaults), `forward` sign
 attributes as `nnAudio.features` v0.3.3 — checked against the unmodified reference by the fixtures in `tests/golden/`
 (signatures, buffers bit-identical for 49 + 7 configurations, attribute surface, exception types, outputs ≤1e-4). What differs:
 
-* inputs must be **CUDA float32** tensors on a B200 (sm_100a); anything else raises — there is no CPU fallback;
+* inputs must be **CUDA** tensors on a B200 (sm_100a); anything else raises — there is no CPU fallback;
+* waveform inputs (`STFT.forward`, `MelSpectrogram`, `MFCC`, `Gammatonegram`, the CQTs, `VQT`, `CFP`) may be float32,
+  **bfloat16 or float16** (the reference's conv1d would reject a 16-bit waveform against its fp32 kernels); the result
+  is float32 and equal to that of the fp32 copy of the same samples, and the input gradient has the input's dtype
+  (DESIGN.md §3.10).  Spectrogram inputs (`iSTFT`, `STFT.inverse`, `Griffin_Lim`) stay float32; other dtypes raise;
 * multi-GPU: one process per GPU (`nnaudio_b200.parallel.BatchShardedTransform`, INTEGRATION.md) is the fast path;
   `torch.nn.DataParallel`, the reference's own mode, also works (per-device launch attributes and caches);
 * `Griffin_Lim.forward(S, rand_phase=None)` takes an optional initial phase (reproducible runs); `device` moves the

@@ -63,6 +63,16 @@ typedef enum nnab_status {
 #define NNAB_FMT_PHASE_ANGLE 2 /* (B, F, T)     atan2(im + 0.0, re)   STFT 'Phase'   */
 #define NNAB_FMT_PHASE_UNIT 3  /* (B, F, T, 2)  (cos, sin)(atan2(im, re)) CQT 'Phase'*/
 
+/* element type of a waveform input `x` (the *_ex entry points).  Outputs stay fp32.  A 16-bit
+ * input gives the same result as its fp32 copy on the same kernel path (every bf16 / fp16 value
+ * is exact in fp32 and in a bf16 hi + lo split); bf16 input lets the tensor-core kernels drop the
+ * x_lo term of the split (two MMAs per K16 slice instead of three). */
+typedef enum nnab_dtype {
+  NNAB_DTYPE_F32 = 0,
+  NNAB_DTYPE_BF16 = 1,
+  NNAB_DTYPE_F16 = 2
+} nnab_dtype;
+
 /* kernel family */
 #define NNAB_PATH_AUTO 0
 #define NNAB_PATH_SIMT 1
@@ -134,6 +144,14 @@ int nnab_stft_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch,
                       int n_fft, int F, int hop, int center, int pad_mode,
                       int out_format, float sqrt_eps, float* out, int64_t T,
                       void* workspace, size_t ws_bytes, int path, void* stream);
+/* Same, for x of element type x_dtype (nnab_dtype); x_pitch in elements.  Every waveform entry
+ * point has such an _ex form; the plain one is the _ex call with NNAB_DTYPE_F32.  The workspace
+ * queries do not depend on the dtype.  An unknown dtype returns NNAB_EINVAL before any device work. */
+int nnab_stft_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch, const float* wcos,
+                         const float* wsin, const void* packed, int n_fft, int F, int hop,
+                         int center, int pad_mode, int out_format, float sqrt_eps, float* out,
+                         int64_t T, void* workspace, size_t ws_bytes, int path, void* stream,
+                         int x_dtype);
 
 /* ------------------------------------------------------------------------- *
  * Banded filterbank table (tcgen05 path): for every FFT bin the (at most two)
@@ -162,6 +180,12 @@ int nnab_stft_filterbank_forward(const float* x, int64_t B, int64_t L, int64_t x
                                  float sqrt_eps, float power, const float* fb, int n_fb,
                                  const void* fb_table, float* out, int64_t T,
                                  void* workspace, size_t ws_bytes, int path, void* stream);
+int nnab_stft_filterbank_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch,
+                                    const float* wcos, const float* wsin, const void* packed,
+                                    int n_fft, int F, int hop, int center, int pad_mode,
+                                    float sqrt_eps, float power, const float* fb, int n_fb,
+                                    const void* fb_table, float* out, int64_t T, void* workspace,
+                                    size_t ws_bytes, int path, void* stream, int x_dtype);
 
 /* ------------------------------------------------------------------------- *
  * MFCC.forward — features/mel.py:309-326 (= mel -> _power_to_db :263-279 ->
@@ -178,6 +202,13 @@ int nnab_mfcc_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch,
                       const void* fb_table, float amin, float ref, float top_db,
                       const float* dct, int n_mfcc, float* out, int64_t T,
                       void* workspace, size_t ws_bytes, int path, void* stream);
+int nnab_mfcc_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch, const float* wcos,
+                         const float* wsin, const void* packed, int n_fft, int F, int hop,
+                         int center, int pad_mode, float sqrt_eps, float power,
+                         const float* mel_basis, int n_mels, const void* fb_table, float amin,
+                         float ref, float top_db, const float* dct, int n_mfcc, float* out,
+                         int64_t T, void* workspace, size_t ws_bytes, int path, void* stream,
+                         int x_dtype);
 
 /* ------------------------------------------------------------------------- *
  * CQT1992v2.forward — features/cqt.py:712-780.
@@ -197,6 +228,13 @@ int nnab_cqt1992v2_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch
                            const float* scale, float scale_all, int out_format,
                            float sqrt_eps, float* out, int64_t T,
                            void* workspace, size_t ws_bytes, int path, void* stream);
+int nnab_cqt1992v2_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch,
+                              const float* k_real, const float* k_imag, const void* packed,
+                              const int32_t* h_k_begin, const int32_t* h_k_end, int n_bins,
+                              int width, int hop, int center, int pad_mode, const float* scale,
+                              float scale_all, int out_format, float sqrt_eps, float* out,
+                              int64_t T, void* workspace, size_t ws_bytes, int path, void* stream,
+                              int x_dtype);
 
 /* ------------------------------------------------------------------------- *
  * CQT2010v2.forward / VQT.forward — features/cqt.py:1070-1139,
@@ -256,6 +294,17 @@ int nnab_cqt_pyramid_forward(const float* x, int64_t B, int64_t L, int64_t x_pit
                              const float* scale, float scale_all, int out_format,
                              float sqrt_eps, float* out, int64_t T,
                              void* workspace, size_t ws_bytes, int path, void* stream);
+/* With a 16-bit x only the first pyramid level reads it (and only level 0's octave runs the
+ * two-term contraction for bf16); the decimated levels are fp32 signals as before. */
+int nnab_cqt_pyramid_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch,
+                                int n_octaves, const float* const* h_k_real,
+                                const float* const* h_k_imag, const void* const* h_packed,
+                                const int32_t* h_widths, int n_filters, const float* lowpass,
+                                const void* lowpass_packed, const float* early_filter,
+                                const void* early_packed, int early_factor, int hop, int pad_mode,
+                                int n_bins, const float* scale, float scale_all, int out_format,
+                                float sqrt_eps, float* out, int64_t T, void* workspace,
+                                size_t ws_bytes, int path, void* stream, int x_dtype);
 
 /* ------------------------------------------------------------------------- *
  * STFT.inverse / iSTFT.forward — features/stft.py:15-63 (inverse_stft), :318-356,

@@ -3,7 +3,8 @@
 PyTorch is used only for device memory and the current CUDA stream; every
 compute call goes through the C ABI with raw device pointers.  There is no
 CPU / eager fallback: if the library is missing, or a tensor is not a CUDA
-fp32 tensor, the call fails loudly.
+tensor of a supported dtype (fp32; waveform inputs also bf16 / fp16), the call
+fails loudly.
 """
 from __future__ import annotations
 
@@ -19,6 +20,10 @@ LIB_PATH = os.path.join(_HERE, "libnnab.so")
 PAD_REFLECT, PAD_CONSTANT = 0, 1
 FMT_MAGNITUDE, FMT_COMPLEX, FMT_PHASE_ANGLE, FMT_PHASE_UNIT = 0, 1, 2, 3
 PATH_AUTO, PATH_SIMT, PATH_TCGEN05 = 0, 1, 2
+DTYPE_F32, DTYPE_BF16, DTYPE_F16 = 0, 1, 2  # nnab_dtype: element type of a waveform input
+
+# waveform element types the forward entry points read (outputs stay fp32)
+X_DTYPES = {torch.float32: DTYPE_F32, torch.bfloat16: DTYPE_BF16, torch.float16: DTYPE_F16}
 
 _PATH_NAMES = {"auto": PATH_AUTO, "simt": PATH_SIMT, "tcgen05": PATH_TCGEN05}
 
@@ -102,6 +107,32 @@ SIGNATURES = {
         c_int, [_P, c_int64, c_int64, c_int64, _P, c_int, c_int, _P, c_int64, _P]),
     "nnab_packed_fir_bytes": (c_size_t, [c_int, c_int]),
     "nnab_pack_fir": (c_int, [_P, c_int, c_int, _P, _P]),
+    "nnab_stft_forward_ex": (
+        c_int,
+        [_P, c_int64, c_int64, c_int64, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_int,
+         c_float, _P, c_int64, _P, c_size_t, c_int, _P, c_int],
+    ),
+    "nnab_stft_filterbank_forward_ex": (
+        c_int,
+        [_P, c_int64, c_int64, c_int64, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float,
+         c_float, _P, c_int, _P, _P, c_int64, _P, c_size_t, c_int, _P, c_int],
+    ),
+    "nnab_mfcc_forward_ex": (
+        c_int,
+        [_P, c_int64, c_int64, c_int64, _P, _P, _P, c_int, c_int, c_int, c_int, c_int, c_float,
+         c_float, _P, c_int, _P, c_float, c_float, c_float, _P, c_int, _P, c_int64, _P, c_size_t,
+         c_int, _P, c_int],
+    ),
+    "nnab_cqt1992v2_forward_ex": (
+        c_int,
+        [_P, c_int64, c_int64, c_int64, _P, _P, _P, _P, _P, c_int, c_int, c_int, c_int, c_int,
+         _P, c_float, c_int, c_float, _P, c_int64, _P, c_size_t, c_int, _P, c_int],
+    ),
+    "nnab_cqt_pyramid_forward_ex": (
+        c_int,
+        [_P, c_int64, c_int64, c_int64, c_int, _P, _P, _P, _P, c_int, _P, _P, _P, _P, c_int, c_int,
+         c_int, c_int, _P, c_float, c_int, c_float, _P, c_int64, _P, c_size_t, c_int, _P, c_int],
+    ),
     "nnab_cqt_pyramid_workspace_bytes": (
         c_size_t, [c_int64, c_int64, c_int, c_int, c_int, c_int, c_int]),
     "nnab_cqt_pyramid_forward": (
@@ -202,6 +233,29 @@ def _dev_f32(t: torch.Tensor, name: str) -> torch.Tensor:
     return t
 
 
+def x_dtype_code(dtype: torch.dtype, name: str = "x") -> int:
+    """nnab_dtype of a waveform input; RuntimeError for any dtype the kernels do not read."""
+    code = X_DTYPES.get(dtype)
+    if code is None:
+        raise RuntimeError(f"{name} must be float32, bfloat16 or float16, got {dtype}")
+    return code
+
+
+def _dev_wave(t: torch.Tensor, name: str) -> int:
+    """A CUDA waveform tensor (fp32, bf16 or fp16) -> its nnab_dtype code."""
+    if isinstance(t, torch.Tensor) and t.dtype == torch.float32:
+        _dev_f32(t, name)  # the fp32 inputs' check, as for every other tensor
+        return DTYPE_F32
+    if not isinstance(t, torch.Tensor):
+        raise TypeError(f"{name} must be a torch.Tensor")
+    if not t.is_cuda:
+        raise RuntimeError(
+            f"{name} is on {t.device}: nnaudio_b200 runs only on CUDA (sm_100a) tensors; "
+            "there is no CPU fallback"
+        )
+    return x_dtype_code(t.dtype, name)
+
+
 def _ptr(t):
     return c_void_p(t.data_ptr()) if t is not None else None
 
@@ -272,14 +326,15 @@ def _batch_chunked(fn):
 
 
 def _rows(x: torch.Tensor):
-    """(B, L) view with unit inner stride -> (tensor, B, L, pitch)."""
-    x = _dev_f32(x, "x")
+    """(B, L) CUDA waveform (fp32, bf16 or fp16) with unit inner stride ->
+    (tensor, B, L, pitch in elements, nnab_dtype code)."""
+    code = _dev_wave(x, "x")
     if x.dim() != 2:
         raise ValueError("internal: expected (B, L)")
     if x.stride(-1) != 1 or (x.shape[0] > 1 and x.stride(0) < x.shape[1]):
         x = x.contiguous()
     pitch = x.stride(0) if x.shape[0] > 1 else x.shape[1]
-    return x, x.shape[0], x.shape[1], pitch
+    return x, x.shape[0], x.shape[1], pitch, code
 
 
 # --------------------------------------------------------------------------- #
@@ -369,7 +424,7 @@ def build_filterbank_table(fb: torch.Tensor):
 def stft_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode, out_format, sqrt_eps,
                  path=None):
     L = lib()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, xdt = _rows(x)
     F = wcos.shape[0]
     pad = n_fft // 2 if center else 0
     T = (Ln + 2 * pad - n_fft) // hop + 1
@@ -379,9 +434,9 @@ def stft_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode, out_format
     with torch.cuda.device(x.device):
         ws, wsb = _workspace(L.nnab_stft_workspace_bytes(B, Ln, n_fft, F, hop, int(center), path),
                              x.device)
-        rc = L.nnab_stft_forward(_ptr(x), B, Ln, pitch, _ptr(wcos), _ptr(wsin), _ptr(packed),
-                                 n_fft, F, hop, int(center), pad_mode, out_format, sqrt_eps,
-                                 _ptr(out), T, _ptr(ws), wsb, path, _stream(x.device))
+        rc = L.nnab_stft_forward_ex(_ptr(x), B, Ln, pitch, _ptr(wcos), _ptr(wsin), _ptr(packed),
+                                    n_fft, F, hop, int(center), pad_mode, out_format, sqrt_eps,
+                                    _ptr(out), T, _ptr(ws), wsb, path, _stream(x.device), xdt)
     _check(rc, "nnab_stft_forward")
     return out
 
@@ -390,7 +445,7 @@ def stft_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode, out_format
 def stft_filterbank_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode, sqrt_eps, power,
                             fb, fb_table=None, path=None):
     L = lib()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, xdt = _rows(x)
     F = wcos.shape[0]
     n_fb = fb.shape[0]
     pad = n_fft // 2 if center else 0
@@ -402,10 +457,10 @@ def stft_filterbank_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode,
             L.nnab_filterbank_workspace_bytes(B, Ln, n_fft, F, hop, int(center), n_fb, path,
                                               int(fb_table is not None)),
             x.device)
-        rc = L.nnab_stft_filterbank_forward(
+        rc = L.nnab_stft_filterbank_forward_ex(
             _ptr(x), B, Ln, pitch, _ptr(wcos), _ptr(wsin), _ptr(packed), n_fft, F, hop,
             int(center), pad_mode, sqrt_eps, power, _ptr(fb), n_fb, _ptr(fb_table), _ptr(out), T,
-            _ptr(ws), wsb, path, _stream(x.device))
+            _ptr(ws), wsb, path, _stream(x.device), xdt)
     _check(rc, "nnab_stft_filterbank_forward")
     return out
 
@@ -414,7 +469,7 @@ def stft_filterbank_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode,
 def mfcc_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode, sqrt_eps, power, mel_basis,
                  amin, ref, top_db, dct, fb_table=None, path=None):
     L = lib()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, xdt = _rows(x)
     F = wcos.shape[0]
     n_mels = mel_basis.shape[0]
     n_mfcc = dct.shape[0]
@@ -426,11 +481,11 @@ def mfcc_forward(x, wcos, wsin, packed, n_fft, hop, center, pad_mode, sqrt_eps, 
         ws, wsb = _workspace(
             L.nnab_mfcc_workspace_bytes(B, Ln, n_fft, F, hop, int(center), n_mels, path,
                                         int(fb_table is not None)), x.device)
-        rc = L.nnab_mfcc_forward(
+        rc = L.nnab_mfcc_forward_ex(
             _ptr(x), B, Ln, pitch, _ptr(wcos), _ptr(wsin), _ptr(packed), n_fft, F, hop,
             int(center), pad_mode, sqrt_eps, power, _ptr(mel_basis), n_mels, _ptr(fb_table), amin, ref,
             -1.0 if top_db is None else float(top_db), _ptr(dct), n_mfcc, _ptr(out), T, _ptr(ws),
-            wsb, path, _stream(x.device))
+            wsb, path, _stream(x.device), xdt)
     _check(rc, "nnab_mfcc_forward")
     return out
 
@@ -440,7 +495,7 @@ def cqt1992v2_forward(x, k_real, k_imag, packed, k_begin, k_end, hop, center, pa
                       scale_all, out_format, sqrt_eps, path=None):
     """k_begin / k_end: host int32 numpy arrays (per-bin support) or None."""
     L = lib()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, xdt = _rows(x)
     n_bins, width = k_real.shape
     pad = width // 2 if center else 0
     T = (Ln + 2 * pad - width) // hop + 1
@@ -453,10 +508,10 @@ def cqt1992v2_forward(x, k_real, k_imag, packed, k_begin, k_end, hop, center, pa
         ws, wsb = _workspace(
             L.nnab_cqt1992v2_workspace_bytes(B, Ln, width, n_bins, hop, int(center), path),
             x.device)
-        rc = L.nnab_cqt1992v2_forward(
+        rc = L.nnab_cqt1992v2_forward_ex(
             _ptr(x), B, Ln, pitch, _ptr(k_real), _ptr(k_imag), _ptr(packed), kb, ke, n_bins,
             width, hop, int(center), pad_mode, _ptr(scale), scale_all, out_format, sqrt_eps,
-            _ptr(out), T, _ptr(ws), wsb, path, _stream(x.device))
+            _ptr(out), T, _ptr(ws), wsb, path, _stream(x.device), xdt)
     _check(rc, "nnab_cqt1992v2_forward")
     return out
 
@@ -468,7 +523,7 @@ def cqt_pyramid_forward(x, banks_real, banks_imag, packed, lowpass, lowpass_pack
     """banks_*: lists (octave 0 = top) of (n_filters, width_i) fp32 CUDA tensors;
     packed: list of packed-basis tensors (or None entries) per octave."""
     L = lib()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, xdt = _rows(x)
     n_oct = len(banks_real)
     n_filters = banks_real[0].shape[0]
     re_arr = (c_void_p * n_oct)(*[t.data_ptr() for t in banks_real])
@@ -483,11 +538,12 @@ def cqt_pyramid_forward(x, banks_real, banks_imag, packed, lowpass, lowpass_pack
         ws, wsb = _workspace(
             L.nnab_cqt_pyramid_workspace_bytes(B, Ln, n_oct, early_factor, max_width, hop, path),
             x.device)
-        rc = L.nnab_cqt_pyramid_forward(
+        rc = L.nnab_cqt_pyramid_forward_ex(
             _ptr(x), B, Ln, pitch, n_oct, re_arr, im_arr, pk_arr, widths, n_filters,
             _ptr(lowpass), _ptr(lowpass_packed), _ptr(early_filter), _ptr(early_packed),
             early_factor, hop, pad_mode, n_bins, _ptr(scale),
-            scale_all, out_format, sqrt_eps, _ptr(out), T, _ptr(ws), wsb, path, _stream(x.device))
+            scale_all, out_format, sqrt_eps, _ptr(out), T, _ptr(ws), wsb, path, _stream(x.device),
+            xdt)
     _check(rc, "nnab_cqt_pyramid_forward")
     return out
 
@@ -530,7 +586,7 @@ def istft_forward(X, packed, window, n_fft, hop, center, length):
 def fir_decimate(x, fir, factor):
     """EXPERIMENTAL: y = conv1d(x, fir, stride=factor, padding=(taps-1)//2) for (B, L) rows."""
     L = lib()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, _ = _rows(_dev_f32(x, "x"))
     fir = _dev_f32(fir, "fir").reshape(-1).contiguous()
     taps = fir.numel()
     half = (taps - 1) // 2
@@ -545,7 +601,7 @@ def fir_decimate(x, fir, factor):
 def fir_decimate_adjoint(g, fir, factor, L_in):
     """EXPERIMENTAL: gradient of fir_decimate w.r.t. its input, (B, Ly) -> (B, L_in)."""
     L = lib()
-    g, B, Ly, pitch = _rows(g)
+    g, B, Ly, pitch, _ = _rows(_dev_f32(g, "grad"))
     fir = _dev_f32(fir, "fir").reshape(-1).contiguous()
     dx = torch.empty((B, L_in), dtype=torch.float32, device=g.device)
     with torch.cuda.device(g.device):
@@ -588,7 +644,7 @@ def framed_backward_weight(g, x, K, hop, center, pad_mode):
     L = lib()
     g = _dev_f32(g, "grad")
     g = g if g.is_contiguous() else g.contiguous()
-    x, B, Ln, pitch = _rows(x)
+    x, B, Ln, pitch, _ = _rows(_dev_f32(x, "x"))
     _, F, T, _ = g.shape
     dw = torch.empty((2 * F, K), dtype=torch.float32, device=g.device)
     with torch.cuda.device(g.device):

@@ -1,6 +1,8 @@
 // Shared declarations for libnnab.so (sm_100a only).
 #pragma once
 
+#include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
@@ -37,6 +39,38 @@ void add_exec_flops(double flops);
       return NNAB_ECUDA;                            \
     }                                               \
   } while (0)
+
+// ---- waveform element types (nnab_dtype) ----------------------------------
+// Every bf16 / fp16 value is exactly representable in fp32, so a kernel that reads 16-bit samples and
+// converts them computes what it computes on the fp32 copy of the same tensor.
+inline bool valid_x_dtype(int x_dtype) {
+  return x_dtype == NNAB_DTYPE_F32 || x_dtype == NNAB_DTYPE_BF16 || x_dtype == NNAB_DTYPE_F16;
+}
+
+__device__ __forceinline__ float ldg_sample(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ldg_sample(const __nv_bfloat16* p) {
+  return __uint_as_float((uint32_t)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
+}
+__device__ __forceinline__ float ldg_sample(const __half* p) {
+  return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
+}
+// eight consecutive 16-bit samples of one 16-byte word, converted to fp32
+__device__ __forceinline__ void unpack8(uint4 w, const __nv_bfloat16*, float* v) {
+  const uint32_t u[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    v[2 * e] = __uint_as_float(u[e] << 16);
+    v[2 * e + 1] = __uint_as_float(u[e] & 0xFFFF0000u);
+  }
+}
+__device__ __forceinline__ void unpack8(uint4 w, const __half*, float* v) {
+  const uint32_t u[4] = {w.x, w.y, w.z, w.w};
+#pragma unroll
+  for (int e = 0; e < 4; ++e) {
+    v[2 * e] = __half2float(__ushort_as_half((unsigned short)(u[e] & 0xFFFFu)));
+    v[2 * e + 1] = __half2float(__ushort_as_half((unsigned short)(u[e] >> 16)));
+  }
+}
 
 // ---- problem description shared by the SIMT and tcgen05 framed kernels ----
 // One "framed complex contraction":
@@ -91,8 +125,9 @@ constexpr int FB_STEP_PAD = 160;  // entries past F (a tile's last chunk may ove
 constexpr int FB_EPI_PARTS = 2;
 
 struct FramedProblem {
-  const float* x;      // (B, L) rows, pitch x_pitch
+  const void* x;       // (B, L) rows, pitch x_pitch (elements of x_dtype)
   int64_t B, L, x_pitch;
+  int x_dtype;         // NNAB_DTYPE_* of x (0 = fp32 in a zero-initialised problem)
   const float* w_re;   // (F, K)
   const float* w_im;   // (F, K)
   int F, K, hop;
@@ -125,6 +160,12 @@ struct FramedProblem {
   int planes_pitch;          // FMT_PLANES: elements per frame row (multiple of 64)
 };
 
+// bf16 input has a zero lo plane: the tensor-core kernels skip its TMA loads and the x_lo * w_hi
+// MMA (two bf16 terms instead of three).  Only for a signal the launcher splits itself from x.
+inline bool two_term(const FramedProblem& p) {
+  return p.x_dtype == NNAB_DTYPE_BF16 && p.presplit == nullptr && p.x != nullptr;
+}
+
 int launch_framed_simt(const FramedProblem& p, cudaStream_t stream);
 
 // tcgen05 path (tc_kernels.cu)
@@ -141,13 +182,16 @@ int tc_pack_basis_layout(const float* w_re, const float* w_im, int F, int K, int
 // split-signal geometry / helpers for callers that manage the planes themselves (pyramid)
 void tc_split_geometry(int64_t B, int64_t L, int K, int hop, int pad, int64_t* t_slots,
                        int64_t* plane_stride, int* hop_eff);
-int tc_pad_split(const float* x, int64_t B, int64_t L, int64_t x_pitch, int K, int hop, int pad,
-                 int pad_mode, void* planes, cudaStream_t stream);
-int tc_pad_split_ex(const float* x, int64_t B, int64_t L, int64_t x_pitch, int pad, int pad_mode,
-                    int64_t clip_pitch, int64_t plane_stride, void* planes, cudaStream_t stream);
+// x_dtype: NNAB_DTYPE_* of x.  hi_only (bf16 input only): write the hi plane alone -- for the
+// two-term kernels, which never read the lo plane.
+int tc_pad_split(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int K, int hop,
+                 int pad, int pad_mode, void* planes, cudaStream_t stream, bool hi_only = false);
+int tc_pad_split_ex(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int pad,
+                    int pad_mode, int64_t clip_pitch, int64_t plane_stride, void* planes,
+                    cudaStream_t stream);
 int tc_zero_slots(void* planes, int64_t B, int64_t clip_pitch, int64_t plane_stride, int64_t keep_lo,
                   int64_t keep_hi, cudaStream_t stream);
-int tc_pad_split2(const float* x, int64_t B, int64_t L, int64_t x_pitch,
+int tc_pad_split2(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch,
                   int K_a, int hop_a, int pad_a, int mode_a, void* planes_a,
                   int K_b, int hop_b, int pad_b, int mode_b, void* planes_b, cudaStream_t stream);
 int tc_zero_margins(void* planes, int64_t B, int64_t L, int K, int hop, int pad, int64_t keep_lo,
@@ -201,8 +245,8 @@ int tc_varn_plan_export(const int32_t* k_begin, const int32_t* k_end, int F, int
 int launch_fir_decimate_adjoint(const float* g, int64_t B, int64_t T, int64_t g_pitch,
                                 const float* fir, int taps, int factor, float* dx, int64_t L,
                                 int64_t dx_pitch, cudaStream_t stream);
-int launch_fir_decimate(const float* x, int64_t B, int64_t L, int64_t x_pitch, const float* fir,
-                        int taps, int factor, float* y, int64_t Ly, int64_t y_pitch,
+int launch_fir_decimate(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch,
+                        const float* fir, int taps, int factor, float* y, int64_t Ly, int64_t y_pitch,
                         cudaStream_t stream);
 
 inline int64_t ceil_div64(int64_t a, int64_t b) { return (a + b - 1) / b; }

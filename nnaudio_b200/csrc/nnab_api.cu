@@ -36,7 +36,7 @@ static inline int64_t frames_of(int64_t L, int K, int hop, int pad) {
   return span < 0 ? 0 : span / hop + 1;
 }
 
-static int check_common(const float* x, int64_t B, int64_t L, int64_t x_pitch, int K, int F,
+static int check_common(const void* x, int64_t B, int64_t L, int64_t x_pitch, int K, int F,
                         int hop, int pad, int pad_mode, int64_t T) {
   if (x == nullptr || B < 0 || L <= 0 || x_pitch < L || K <= 0 || F <= 0 || hop <= 0)
     return NNAB_EINVAL;
@@ -254,6 +254,17 @@ int nnab_stft_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch, con
                       const float* wsin, const void* packed, int n_fft, int F, int hop,
                       int center, int pad_mode, int out_format, float sqrt_eps, float* out,
                       int64_t T, void* workspace, size_t ws_bytes, int path, void* stream) {
+  return nnab_stft_forward_ex(x, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, center, pad_mode,
+                              out_format, sqrt_eps, out, T, workspace, ws_bytes, path, stream,
+                              NNAB_DTYPE_F32);
+}
+
+int nnab_stft_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch, const float* wcos,
+                         const float* wsin, const void* packed, int n_fft, int F, int hop,
+                         int center, int pad_mode, int out_format, float sqrt_eps, float* out,
+                         int64_t T, void* workspace, size_t ws_bytes, int path, void* stream,
+                         int x_dtype) {
+  if (!valid_x_dtype(x_dtype)) return NNAB_EINVAL;
   const int pad = center ? n_fft / 2 : 0;
   int rc = check_common(x, B, L, x_pitch, n_fft, F, hop, pad, pad_mode, T);
   if (rc) return rc;
@@ -263,7 +274,7 @@ int nnab_stft_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch, con
     return NNAB_EINVAL;
   if ((rc = check_arch())) return rc;
   FramedProblem p{};
-  p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch;
+  p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch; p.x_dtype = x_dtype;
   p.w_re = wcos; p.w_im = wsin; p.F = F; p.K = n_fft; p.hop = hop;
   p.pad = pad; p.pad_mode = pad_mode; p.scale = nullptr; p.scale_all = 1.f;
   p.fmt = out_format; p.eps = sqrt_eps; p.power = 1.f; p.out = out; p.T = T;
@@ -372,13 +383,13 @@ size_t nnab_filterbank_workspace_bytes(int64_t B, int64_t L, int n_fft, int F, i
   return n;
 }
 
-static int power_spectrogram(const float* x, int64_t B, int64_t L, int64_t x_pitch,
+static int power_spectrogram(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch,
                              const float* wcos, const float* wsin, const void* packed,
                              int n_fft, int F, int hop, int pad, int pad_mode, float sqrt_eps,
                              float power, float* P, int64_t T, void* tc_ws, size_t tc_ws_bytes,
                              int path, cudaStream_t stream) {
   FramedProblem p{};
-  p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch;
+  p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch; p.x_dtype = x_dtype;
   p.w_re = wcos; p.w_im = wsin; p.F = F; p.K = n_fft; p.hop = hop;
   p.pad = pad; p.pad_mode = pad_mode; p.scale = nullptr; p.scale_all = 1.f;
   p.fmt = FMT_POWER; p.eps = sqrt_eps; p.power = power; p.out = P; p.T = T;
@@ -392,6 +403,18 @@ int nnab_stft_filterbank_forward(const float* x, int64_t B, int64_t L, int64_t x
                                  float sqrt_eps, float power, const float* fb, int n_fb,
                                  const void* fb_table, float* out, int64_t T, void* workspace,
                                  size_t ws_bytes, int path, void* stream) {
+  return nnab_stft_filterbank_forward_ex(x, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, center,
+                                         pad_mode, sqrt_eps, power, fb, n_fb, fb_table, out, T,
+                                         workspace, ws_bytes, path, stream, NNAB_DTYPE_F32);
+}
+
+int nnab_stft_filterbank_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch,
+                                    const float* wcos, const float* wsin, const void* packed,
+                                    int n_fft, int F, int hop, int center, int pad_mode,
+                                    float sqrt_eps, float power, const float* fb, int n_fb,
+                                    const void* fb_table, float* out, int64_t T, void* workspace,
+                                    size_t ws_bytes, int path, void* stream, int x_dtype) {
+  if (!valid_x_dtype(x_dtype)) return NNAB_EINVAL;
   const int pad = center ? n_fft / 2 : 0;
   int rc = check_common(x, B, L, x_pitch, n_fft, F, hop, pad, pad_mode, T);
   if (rc) return rc;
@@ -402,7 +425,7 @@ int nnab_stft_filterbank_forward(const float* x, int64_t B, int64_t L, int64_t x
   bool fused = fused_fbank(path, packed, fb_table, n_fft, hop);
   if (fused) {
     FramedProblem p{};
-    p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch;
+    p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch; p.x_dtype = x_dtype;
     p.w_re = wcos; p.w_im = wsin; p.F = F; p.K = n_fft; p.hop = hop;
     p.pad = pad; p.pad_mode = pad_mode; p.scale = nullptr; p.scale_all = 1.f;
     p.fmt = FMT_FBANK; p.eps = sqrt_eps; p.power = power; p.out = out; p.T = T;
@@ -441,7 +464,7 @@ int nnab_stft_filterbank_forward(const float* x, int64_t B, int64_t L, int64_t x
                                         (size_t)(fp.kp - fp.nb * fp.n_tiles) * 2, (size_t)(2 * fp.rows), s));
       // 1. STFT -> |X| ** power as operand planes (block-partial kernel, FMT_PLANES)
       FramedProblem p{};
-      p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch;
+      p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch; p.x_dtype = x_dtype;
       p.w_re = wcos; p.w_im = wsin; p.F = F; p.K = n_fft; p.hop = hop;
       p.pad = pad; p.pad_mode = pad_mode; p.scale = nullptr; p.scale_all = 1.f;
       p.fmt = FMT_PLANES; p.eps = sqrt_eps; p.power = power; p.out = reinterpret_cast<float*>(planes); p.T = T;
@@ -461,7 +484,7 @@ int nnab_stft_filterbank_forward(const float* x, int64_t B, int64_t L, int64_t x
   }
   float* P = (float*)workspace;
   const size_t pb = power_bytes(B, F, T);
-  rc = power_spectrogram(x, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, pad, pad_mode,
+  rc = power_spectrogram(x, x_dtype, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, pad, pad_mode,
                          sqrt_eps, power, P, T, (char*)workspace + pb, ws_bytes - pb, path, s);
   if (rc) return rc;
   return launch_filterbank(P, fb, B, F, T, n_fb, out, s);
@@ -487,6 +510,19 @@ int nnab_mfcc_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch, con
                       const float* mel_basis, int n_mels, const void* fb_table, float amin,
                       float ref, float top_db, const float* dct, int n_mfcc, float* out,
                       int64_t T, void* workspace, size_t ws_bytes, int path, void* stream) {
+  return nnab_mfcc_forward_ex(x, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, center, pad_mode,
+                              sqrt_eps, power, mel_basis, n_mels, fb_table, amin, ref, top_db, dct,
+                              n_mfcc, out, T, workspace, ws_bytes, path, stream, NNAB_DTYPE_F32);
+}
+
+int nnab_mfcc_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch, const float* wcos,
+                         const float* wsin, const void* packed, int n_fft, int F, int hop,
+                         int center, int pad_mode, float sqrt_eps, float power,
+                         const float* mel_basis, int n_mels, const void* fb_table, float amin,
+                         float ref, float top_db, const float* dct, int n_mfcc, float* out,
+                         int64_t T, void* workspace, size_t ws_bytes, int path, void* stream,
+                         int x_dtype) {
+  if (!valid_x_dtype(x_dtype)) return NNAB_EINVAL;
   const int pad = center ? n_fft / 2 : 0;
   int rc = check_common(x, B, L, x_pitch, n_fft, F, hop, pad, pad_mode, T);
   if (rc) return rc;
@@ -500,9 +536,9 @@ int nnab_mfcc_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch, con
       align_up(nnab_filterbank_workspace_bytes(B, L, n_fft, F, hop, center, n_mels, path, 0), 256);
   float* mel = (float*)((char*)workspace + fbw);
   unsigned int* scratch = (unsigned int*)((char*)workspace + fbw + mel_bytes(B, n_mels, T));
-  rc = nnab_stft_filterbank_forward(x, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, center,
-                                    pad_mode, sqrt_eps, power, mel_basis, n_mels, fb_table, mel,
-                                    T, workspace, fbw, path, stream);
+  rc = nnab_stft_filterbank_forward_ex(x, B, L, x_pitch, wcos, wsin, packed, n_fft, F, hop, center,
+                                       pad_mode, sqrt_eps, power, mel_basis, n_mels, fb_table, mel,
+                                       T, workspace, fbw, path, stream, x_dtype);
   if (rc) return rc;
   return launch_mfcc_tail(mel, B, n_mels, T, amin, ref, top_db, dct, n_mfcc, out, scratch,
                           (cudaStream_t)stream);
@@ -524,6 +560,19 @@ int nnab_cqt1992v2_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch
                            float scale_all, int out_format, float sqrt_eps, float* out,
                            int64_t T, void* workspace, size_t ws_bytes, int path,
                            void* stream) {
+  return nnab_cqt1992v2_forward_ex(x, B, L, x_pitch, k_real, k_imag, packed, h_k_begin, h_k_end, n_bins,
+                                   width, hop, center, pad_mode, scale, scale_all, out_format, sqrt_eps,
+                                   out, T, workspace, ws_bytes, path, stream, NNAB_DTYPE_F32);
+}
+
+int nnab_cqt1992v2_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch,
+                              const float* k_real, const float* k_imag, const void* packed,
+                              const int32_t* h_k_begin, const int32_t* h_k_end, int n_bins,
+                              int width, int hop, int center, int pad_mode, const float* scale,
+                              float scale_all, int out_format, float sqrt_eps, float* out,
+                              int64_t T, void* workspace, size_t ws_bytes, int path, void* stream,
+                              int x_dtype) {
+  if (!valid_x_dtype(x_dtype)) return NNAB_EINVAL;
   const int pad = center ? width / 2 : 0;
   int rc = check_common(x, B, L, x_pitch, width, n_bins, hop, pad, pad_mode, T);
   if (rc) return rc;
@@ -533,7 +582,7 @@ int nnab_cqt1992v2_forward(const float* x, int64_t B, int64_t L, int64_t x_pitch
     return NNAB_EINVAL;
   if ((rc = check_arch())) return rc;
   FramedProblem p{};
-  p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch;
+  p.x = x; p.B = B; p.L = L; p.x_pitch = x_pitch; p.x_dtype = x_dtype;
   p.w_re = k_real; p.w_im = k_imag; p.F = n_bins; p.K = width; p.hop = hop;
   p.pad = pad; p.pad_mode = pad_mode; p.scale = scale; p.scale_all = scale_all;
   p.fmt = out_format; p.eps = sqrt_eps; p.power = 1.f; p.out = out; p.T = T;
@@ -722,7 +771,8 @@ int nnab_fir_decimate(const float* x, int64_t B, int64_t L, int64_t x_pitch, con
     return NNAB_EINVAL;
   int rc = check_arch();
   if (rc) return rc;
-  return launch_fir_decimate(x, B, L, x_pitch, fir, taps, factor, y, Ly, Ly, (cudaStream_t)stream);
+  return launch_fir_decimate(x, NNAB_DTYPE_F32, B, L, x_pitch, fir, taps, factor, y, Ly, Ly,
+                             (cudaStream_t)stream);
 }
 
 int nnab_fir_decimate_adjoint(const float* g, int64_t B, int64_t Ly, int64_t g_pitch,
@@ -765,7 +815,7 @@ size_t nnab_cqt_pyramid_workspace_bytes(int64_t B, int64_t L, int n_octaves, int
   return n;
 }
 
-static int pyramid_fused2(const float* x, int64_t B, int64_t L, int64_t x_pitch, int n_octaves,
+static int pyramid_fused2(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int n_octaves,
                           const float* const* h_k_real, const float* const* h_k_imag,
                           const void* const* h_packed, const int32_t* h_widths, int n_filters,
                           const float* lowpass, const void* lowpass_packed, int hop, int pad_mode,
@@ -790,9 +840,10 @@ static int pyramid_fused2(const float* x, int64_t B, int64_t L, int64_t x_pitch,
   int rc;
   const size_t scratch_bytes = ws_bytes - 256 - scratch_off;
 
-  // level 0: the caller's fp32 waveform -> planes (one pass; writes the whole clip slot)
+  // level 0: the caller's waveform -> planes (one pass; writes the whole clip slot, both planes: the
+  // octave and FIR kernels run the three-term split whatever the input type)
   if (lv[0].planes) {
-    rc = tc_pad_split_ex(x, B, L, x_pitch, lv[0].pad, lv[0].mode, lv[0].pitch, lv[0].plane,
+    rc = tc_pad_split_ex(x, x_dtype, B, L, x_pitch, lv[0].pad, lv[0].mode, lv[0].pitch, lv[0].plane,
                          ws + lv[0].pc, s);
     if (rc) return rc;
   }
@@ -822,8 +873,9 @@ static int pyramid_fused2(const float* x, int64_t B, int64_t L, int64_t x_pitch,
       }
       if (!done && (rc = run_framed(p, h_packed[i], nullptr, 0, NNAB_PATH_TCGEN05, s))) return rc;
     } else {
-      const float* src = (i == 0) ? x : (const float*)(ws + l.y32);
-      p.x = src; p.x_pitch = (i == 0) ? x_pitch : l.y32_pitch;
+      p.x = (i == 0) ? x : (const void*)(ws + l.y32);
+      p.x_pitch = (i == 0) ? x_pitch : l.y32_pitch;
+      p.x_dtype = (i == 0) ? x_dtype : NNAB_DTYPE_F32;
       if ((rc = run_framed(p, h_packed[i], scratch, scratch_bytes, NNAB_PATH_TCGEN05, s))) return rc;
     }
     if (i == n_octaves - 1) break;
@@ -850,7 +902,7 @@ static int pyramid_fused2(const float* x, int64_t B, int64_t L, int64_t x_pitch,
 
 // All-tensor-core pyramid; returns NNAB_EUNSUPPORTED when the plan cannot be used (the caller
 // then takes the per-octave path).
-static int pyramid_fused(const float* x, int64_t B, int64_t L, int64_t x_pitch, int n_octaves,
+static int pyramid_fused(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int n_octaves,
                          const float* const* h_k_real, const float* const* h_k_imag,
                          const void* const* h_packed, const int32_t* h_widths, int n_filters,
                          const void* lowpass_packed, const void* early_packed, int early_factor,
@@ -919,28 +971,30 @@ static int pyramid_fused(const float* x, int64_t B, int64_t L, int64_t x_pitch, 
   };
 
   // ---- level 0 ------------------------------------------------------------------------
-  const float* x0 = x;         // fp32 level-0 signal when available
+  const void* x0 = x;          // level-0 signal when available (x0_dtype)
   int64_t x0_pitch = x_pitch;
+  int x0_dtype = x_dtype;
   if (early_factor > 1) {
-    rc = tc_pad_split(x, B, L, x_pitch, tc_fir_k(FIR_TAPS, early_factor), 128 * early_factor,
+    rc = tc_pad_split(x, x_dtype, B, L, x_pitch, tc_fir_k(FIR_TAPS, early_factor), 128 * early_factor,
                       FIR_OFF, NNAB_PAD_CONSTANT, ws + pf_early, s);
     if (rc) return rc;
     if ((rc = fir_stage(ws + pf_early, L, early_factor, early_packed, lv[0]))) return rc;
-    x0 = lv[0].y32 != SIZE_MAX ? (const float*)(ws + lv[0].y32) : nullptr;
+    x0 = lv[0].y32 != SIZE_MAX ? (const void*)(ws + lv[0].y32) : nullptr;
     x0_pitch = lv[0].y32_pitch;
+    x0_dtype = NNAB_DTYPE_F32;
   } else {
     if (lv[0].pc != SIZE_MAX && lv[0].pf != SIZE_MAX) {
       // one pass over x: reflect-padded copy for the octave CQT + zero-margin copy for the FIR
-      rc = tc_pad_split2(x, B, L, x_pitch, lv[0].width, lv[0].hop, lv[0].pad, lv[0].mode,
+      rc = tc_pad_split2(x, x_dtype, B, L, x_pitch, lv[0].width, lv[0].hop, lv[0].pad, lv[0].mode,
                          ws + lv[0].pc, tc_fir_k(FIR_TAPS, 2), 256, FIR_OFF, NNAB_PAD_CONSTANT,
                          ws + lv[0].pf, s);
       if (rc) return rc;
     } else if (lv[0].pc != SIZE_MAX) {
-      rc = tc_pad_split(x, B, L, x_pitch, lv[0].width, lv[0].hop, lv[0].pad, lv[0].mode,
+      rc = tc_pad_split(x, x_dtype, B, L, x_pitch, lv[0].width, lv[0].hop, lv[0].pad, lv[0].mode,
                         ws + lv[0].pc, s);
       if (rc) return rc;
     } else if (lv[0].pf != SIZE_MAX) {
-      rc = tc_pad_split(x, B, L, x_pitch, tc_fir_k(FIR_TAPS, 2), 256, FIR_OFF, NNAB_PAD_CONSTANT,
+      rc = tc_pad_split(x, x_dtype, B, L, x_pitch, tc_fir_k(FIR_TAPS, 2), 256, FIR_OFF, NNAB_PAD_CONSTANT,
                         ws + lv[0].pf, s);
       if (rc) return rc;
     }
@@ -961,10 +1015,11 @@ static int pyramid_fused(const float* x, int64_t B, int64_t L, int64_t x_pitch, 
       p.x = nullptr; p.x_pitch = 0; p.presplit = ws + l.pc;
       if ((rc = run_framed(p, h_packed[i], nullptr, 0, NNAB_PATH_TCGEN05, s))) return rc;
     } else {
-      const float* src = (i == 0) ? x0 : (const float*)(ws + l.y32);
+      const void* src = (i == 0) ? x0 : (const void*)(ws + l.y32);
       const int64_t pitch = (i == 0) ? x0_pitch : l.y32_pitch;
       if (src == nullptr) return NNAB_EINVAL;
       p.x = src; p.x_pitch = pitch; p.presplit = nullptr;
+      p.x_dtype = (i == 0) ? x0_dtype : NNAB_DTYPE_F32;
       if ((rc = run_framed(p, h_packed[i], scratch, scratch_bytes, NNAB_PATH_TCGEN05, s))) return rc;
     }
     if (i < n_octaves - 1)
@@ -982,6 +1037,22 @@ int nnab_cqt_pyramid_forward(const float* x, int64_t B, int64_t L, int64_t x_pit
                              const float* scale, float scale_all, int out_format, float sqrt_eps,
                              float* out, int64_t T, void* workspace, size_t ws_bytes, int path,
                              void* stream) {
+  return nnab_cqt_pyramid_forward_ex(x, B, L, x_pitch, n_octaves, h_k_real, h_k_imag, h_packed, h_widths,
+                                     n_filters, lowpass, lowpass_packed, early_filter, early_packed,
+                                     early_factor, hop, pad_mode, n_bins, scale, scale_all, out_format,
+                                     sqrt_eps, out, T, workspace, ws_bytes, path, stream, NNAB_DTYPE_F32);
+}
+
+int nnab_cqt_pyramid_forward_ex(const void* x, int64_t B, int64_t L, int64_t x_pitch, int n_octaves,
+                                const float* const* h_k_real, const float* const* h_k_imag,
+                                const void* const* h_packed, const int32_t* h_widths, int n_filters,
+                                const float* lowpass, const void* lowpass_packed,
+                                const float* early_filter, const void* early_packed,
+                                int early_factor, int hop, int pad_mode, int n_bins,
+                                const float* scale, float scale_all, int out_format, float sqrt_eps,
+                                float* out, int64_t T, void* workspace, size_t ws_bytes, int path,
+                                void* stream, int x_dtype) {
+  if (!valid_x_dtype(x_dtype)) return NNAB_EINVAL;
   if (x == nullptr || out == nullptr || h_k_real == nullptr || h_k_imag == nullptr ||
       h_widths == nullptr || lowpass == nullptr || B < 0 || L <= 0 || x_pitch < L ||
       n_octaves <= 0 || n_filters <= 0 || hop <= 0 || n_bins <= 0 || early_factor < 1)
@@ -1006,13 +1077,13 @@ int nnab_cqt_pyramid_forward(const float* x, int64_t B, int64_t L, int64_t x_pit
   for (int i = 0; all_packed && i < n_octaves; ++i) all_packed = h_packed[i] != nullptr;
   if (all_packed && getenv("NNAB_PYRAMID_UNFUSED") == nullptr && early_factor <= 1 &&
       !(getenv("NNAB_PYRAMID2") != nullptr && atoi(getenv("NNAB_PYRAMID2")) == 0)) {
-    rc = pyramid_fused2(x, B, L, x_pitch, n_octaves, h_k_real, h_k_imag, h_packed, h_widths, n_filters,
+    rc = pyramid_fused2(x, x_dtype, B, L, x_pitch, n_octaves, h_k_real, h_k_imag, h_packed, h_widths, n_filters,
                         lowpass, lowpass_packed, hop, pad_mode, n_bins, scale, scale_all, out_format,
                         sqrt_eps, out, T, workspace, ws_bytes, s);
     if (rc != NNAB_EUNSUPPORTED) return rc;
   }
   if (all_packed && getenv("NNAB_PYRAMID_UNFUSED") == nullptr) {
-    rc = pyramid_fused(x, B, L, x_pitch, n_octaves, h_k_real, h_k_imag, h_packed, h_widths,
+    rc = pyramid_fused(x, x_dtype, B, L, x_pitch, n_octaves, h_k_real, h_k_imag, h_packed, h_widths,
                        n_filters, lowpass_packed, early_packed, early_factor, hop, pad_mode, n_bins,
                        scale, scale_all, out_format, sqrt_eps, out, T, workspace, ws_bytes, s);
     if (rc != NNAB_EUNSUPPORTED) return rc;
@@ -1023,17 +1094,18 @@ int nnab_cqt_pyramid_forward(const float* x, int64_t B, int64_t L, int64_t x_pit
   char* tc_ws = (char*)workspace + level_bytes;
   const size_t tc_ws_bytes = ws_bytes - level_bytes;
   char* wsp = (char*)workspace;
-  const float* cur = x;
+  const void* cur = x;  // level signal: x (x_dtype) at level 0, fp32 below
+  int cur_dtype = x_dtype;
   int64_t cur_len = L, cur_pitch = x_pitch;
   if (early_factor > 1) {
     const int64_t L0 = decimated_len(L, early_factor);
     const int64_t pitch0 = (int64_t)align_up((size_t)L0, 4);
     float* e = (float*)wsp;
     wsp += align_up((size_t)B * pitch0 * sizeof(float), 256);
-    if ((rc = launch_fir_decimate(x, B, L, x_pitch, early_filter, 256, early_factor, e, L0,
+    if ((rc = launch_fir_decimate(x, x_dtype, B, L, x_pitch, early_filter, 256, early_factor, e, L0,
                                   pitch0, s)))
       return rc;
-    cur = e; cur_len = L0; cur_pitch = pitch0;
+    cur = e; cur_dtype = NNAB_DTYPE_F32; cur_len = L0; cur_pitch = pitch0;
   }
   const int64_t half_pitch = (int64_t)align_up((size_t)(cur_len / 2 + 1), 4);
   float* pingpong[2];
@@ -1045,10 +1117,10 @@ int nnab_cqt_pyramid_forward(const float* x, int64_t B, int64_t L, int64_t x_pit
     if (i > 0) {
       const int64_t nl = decimated_len(cur_len, 2);
       float* dst = pingpong[i & 1];
-      if ((rc = launch_fir_decimate(cur, B, cur_len, cur_pitch, lowpass, 256, 2, dst, nl,
+      if ((rc = launch_fir_decimate(cur, cur_dtype, B, cur_len, cur_pitch, lowpass, 256, 2, dst, nl,
                                     half_pitch, s)))
         return rc;
-      cur = dst; cur_len = nl; cur_pitch = half_pitch;
+      cur = dst; cur_dtype = NNAB_DTYPE_F32; cur_len = nl; cur_pitch = half_pitch;
       cur_hop /= 2;
     }
     if (cur_hop <= 0 || cur_len <= 0) return NNAB_EINVAL;
@@ -1059,7 +1131,7 @@ int nnab_cqt_pyramid_forward(const float* x, int64_t B, int64_t L, int64_t x_pit
     if (mode == NNAB_PAD_REFLECT && pad >= cur_len) mode = NNAB_PAD_CONSTANT;
     if (frames_of(cur_len, width, cur_hop, pad) != T) return NNAB_EINVAL;
     FramedProblem p{};
-    p.x = cur; p.B = B; p.L = cur_len; p.x_pitch = cur_pitch;
+    p.x = cur; p.B = B; p.L = cur_len; p.x_pitch = cur_pitch; p.x_dtype = cur_dtype;
     p.w_re = h_k_real[i]; p.w_im = h_k_imag[i]; p.F = n_filters; p.K = width; p.hop = cur_hop;
     p.pad = pad; p.pad_mode = mode; p.scale = nullptr; p.scale_all = scale_all;
     p.fmt = out_format; p.eps = sqrt_eps; p.power = 1.f; p.out = out; p.T = T;

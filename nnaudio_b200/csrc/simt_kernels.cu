@@ -14,7 +14,8 @@ namespace nnab {
 // sample fetch with the centre padding folded into the index
 // (nn.ReflectionPad1d / nn.ConstantPad1d semantics, stft.py:278-289)
 // --------------------------------------------------------------------------
-__device__ __forceinline__ float fetch_padded(const float* __restrict__ xb, int64_t L, int64_t j,
+template <typename T>
+__device__ __forceinline__ float fetch_padded(const T* __restrict__ xb, int64_t L, int64_t j,
                                               int pad_mode) {
   if (j < 0) {
     if (pad_mode == NNAB_PAD_CONSTANT) return 0.f;
@@ -23,7 +24,7 @@ __device__ __forceinline__ float fetch_padded(const float* __restrict__ xb, int6
     if (pad_mode == NNAB_PAD_CONSTANT) return 0.f;
     j = 2 * (L - 1) - j;
   }
-  return (j >= 0 && j < L) ? __ldg(xb + j) : 0.f;
+  return (j >= 0 && j < L) ? ldg_sample(xb + j) : 0.f;
 }
 
 // --------------------------------------------------------------------------
@@ -33,7 +34,7 @@ __device__ __forceinline__ float fetch_padded(const float* __restrict__ xb, int6
 constexpr int SIMT_MAX_BIN_TILES = 128;
 
 struct SimtParams {
-  const float* x;
+  const void* x;  // element type: the kernel's T
   int64_t L, x_pitch;
   const float* w_re;
   const float* w_im;
@@ -44,7 +45,7 @@ struct SimtParams {
   EpiParams epi;
 };
 
-template <int TN>
+template <int TN, typename T>
 __global__ void __launch_bounds__(256) framed_cplx_simt_kernel(const SimtParams p) {
   constexpr int TM = 8, BM = 128, BNB = 16 * TN, BK = 16;
   __shared__ float As[BM][BK + 1];
@@ -57,7 +58,7 @@ __global__ void __launch_bounds__(256) framed_cplx_simt_kernel(const SimtParams 
   const int64_t b = blockIdx.z;
   const int64_t t0 = (int64_t)blockIdx.x * BM;
   const int f0 = blockIdx.y * BNB;
-  const float* __restrict__ xb = p.x + b * p.x_pitch;
+  const T* __restrict__ xb = static_cast<const T*>(p.x) + b * p.x_pitch;
 
   int kbeg = 0, kend = p.K;
   if (p.n_ranges > 0) {
@@ -169,10 +170,21 @@ int launch_framed_simt(const FramedProblem& q, cudaStream_t stream) {
     }
   }
   dim3 grid((unsigned)ceil_div64(q.T, 128), (unsigned)n_tiles, (unsigned)q.B);
-  if (TN == 4)
-    framed_cplx_simt_kernel<4><<<grid, 256, 0, stream>>>(p);
-  else
-    framed_cplx_simt_kernel<2><<<grid, 256, 0, stream>>>(p);
+  switch (q.x_dtype) {
+    case NNAB_DTYPE_F32:
+      if (TN == 4) framed_cplx_simt_kernel<4, float><<<grid, 256, 0, stream>>>(p);
+      else framed_cplx_simt_kernel<2, float><<<grid, 256, 0, stream>>>(p);
+      break;
+    case NNAB_DTYPE_BF16:
+      if (TN == 4) framed_cplx_simt_kernel<4, __nv_bfloat16><<<grid, 256, 0, stream>>>(p);
+      else framed_cplx_simt_kernel<2, __nv_bfloat16><<<grid, 256, 0, stream>>>(p);
+      break;
+    case NNAB_DTYPE_F16:
+      if (TN == 4) framed_cplx_simt_kernel<4, __half><<<grid, 256, 0, stream>>>(p);
+      else framed_cplx_simt_kernel<2, __half><<<grid, 256, 0, stream>>>(p);
+      break;
+    default: return NNAB_EINVAL;
+  }
   NNAB_LAUNCH_CHECK();
   return NNAB_OK;
 }
@@ -505,8 +517,9 @@ int launch_mfcc_tail(const float* mel, int64_t B, int n_mels, int64_t T, float a
 //   Polyphase in shared memory so a thread's 4 consecutive outputs slide over
 //   unit-stride data: 2 LDS.128 per 16 FMAs.
 // --------------------------------------------------------------------------
+template <typename T>
 __global__ void __launch_bounds__(256) fir_decimate_kernel(
-    const float* __restrict__ x, int64_t L, int64_t x_pitch, const float* __restrict__ fir,
+    const T* __restrict__ x, int64_t L, int64_t x_pitch, const float* __restrict__ fir,
     int taps, int factor, int qtaps, int ph_len, float* __restrict__ y, int64_t Ly,
     int64_t y_pitch) {
   extern __shared__ __align__(16) float fsm[];
@@ -516,11 +529,11 @@ __global__ void __launch_bounds__(256) fir_decimate_kernel(
   const int64_t b = blockIdx.y;
   const int64_t n0 = (int64_t)blockIdx.x * 1024;
   const int64_t base = n0 * factor - (taps - 1) / 2;
-  const float* __restrict__ xb = x + b * x_pitch;
+  const T* __restrict__ xb = x + b * x_pitch;
 
   for (int idx = tid; idx < ph_len * factor; idx += 256) {
     const int64_t g = base + idx;
-    const float v = (g >= 0 && g < L) ? __ldg(xb + g) : 0.f;
+    const float v = (g >= 0 && g < L) ? ldg_sample(xb + g) : 0.f;
     xs[(idx % factor) * ph_len + idx / factor] = v;
   }
   for (int j = tid; j < qtaps * factor; j += 256)
@@ -554,9 +567,10 @@ __global__ void __launch_bounds__(256) fir_decimate_kernel(
   }
 }
 
-int launch_fir_decimate(const float* x, int64_t B, int64_t L, int64_t x_pitch, const float* fir,
-                        int taps, int factor, float* y, int64_t Ly, int64_t y_pitch,
-                        cudaStream_t stream) {
+template <typename T>
+static int launch_fir_decimate_t(const T* x, int64_t B, int64_t L, int64_t x_pitch, const float* fir,
+                                 int taps, int factor, float* y, int64_t Ly, int64_t y_pitch,
+                                 cudaStream_t stream) {
   if (B <= 0 || Ly <= 0) return NNAB_OK;
   if (B > 65535 || factor < 1 || taps < 1) return NNAB_EUNSUPPORTED;
   int qtaps = (taps + factor - 1) / factor;
@@ -565,13 +579,28 @@ int launch_fir_decimate(const float* x, int64_t B, int64_t L, int64_t x_pitch, c
   const size_t smem = (size_t)factor * (ph_len + qtaps) * sizeof(float);
   if (smem > 200 * 1024) return NNAB_EUNSUPPORTED;
   if (smem > 48 * 1024)
-    NNAB_CUDA_TRY(cudaFuncSetAttribute(fir_decimate_kernel,
+    NNAB_CUDA_TRY(cudaFuncSetAttribute(fir_decimate_kernel<T>,
                                        cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   dim3 grid((unsigned)ceil_div64(Ly, 1024), (unsigned)B);
-  fir_decimate_kernel<<<grid, 256, smem, stream>>>(x, L, x_pitch, fir, taps, factor, qtaps,
-                                                   ph_len, y, Ly, y_pitch);
+  fir_decimate_kernel<T><<<grid, 256, smem, stream>>>(x, L, x_pitch, fir, taps, factor, qtaps,
+                                                      ph_len, y, Ly, y_pitch);
   NNAB_LAUNCH_CHECK();
   return NNAB_OK;
+}
+
+int launch_fir_decimate(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch,
+                        const float* fir, int taps, int factor, float* y, int64_t Ly, int64_t y_pitch,
+                        cudaStream_t stream) {
+  switch (x_dtype) {
+    case NNAB_DTYPE_F32:
+      return launch_fir_decimate_t((const float*)x, B, L, x_pitch, fir, taps, factor, y, Ly, y_pitch, stream);
+    case NNAB_DTYPE_BF16:
+      return launch_fir_decimate_t((const __nv_bfloat16*)x, B, L, x_pitch, fir, taps, factor, y, Ly, y_pitch,
+                                   stream);
+    case NNAB_DTYPE_F16:
+      return launch_fir_decimate_t((const __half*)x, B, L, x_pitch, fir, taps, factor, y, Ly, y_pitch, stream);
+    default: return NNAB_EINVAL;
+  }
 }
 
 // --------------------------------------------------------------------------

@@ -102,43 +102,64 @@ bool tc_supported(const FramedProblem& p) {
 // pre-pass kernels
 // ---------------------------------------------------------------------------
 
-// One thread = 8 consecutive samples of one clip's slot region (16-byte stores).
-__global__ void __launch_bounds__(256) pad_split_kernel(
-    const float* __restrict__ x, int64_t L, int64_t x_pitch, int pad, int pad_mode, int shift,
-    int64_t clip_pitch, int64_t plane_stride, __nv_bfloat16* __restrict__ planes) {
-  const int64_t b = blockIdx.y;
-  const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 8;
-  if (i0 >= clip_pitch) return;
-  const float* __restrict__ xb = x + b * x_pitch;
+// Eight consecutive samples i0 .. i0 + 7 of a centre-padded clip (reflect / zero padding folded
+// into the index).  16-bit input: one 16-byte load when the eight are interior and aligned.
+template <typename T>
+__device__ __forceinline__ void fetch8_padded(const T* __restrict__ xb, int64_t L, int64_t i0,
+                                              int pad, int pad_mode, float* v) {
   const int64_t padded_len = L + 2 * (int64_t)pad;
-  __align__(16) __nv_bfloat16 hi[8];
-  __align__(16) __nv_bfloat16 lo[8];
+  if constexpr (sizeof(T) == 2) {
+    const int64_t j0 = i0 - pad;
+    if (j0 >= 0 && j0 + 8 <= L && ((reinterpret_cast<uintptr_t>(xb + j0) & 15u) == 0)) {
+      unpack8(__ldg(reinterpret_cast<const uint4*>(xb + j0)), xb, v);
+      return;
+    }
+  }
 #pragma unroll
   for (int e = 0; e < 8; ++e) {
-    const int64_t i = i0 + e + shift;  // index into the centre-padded clip
-    float v = 0.f;
+    const int64_t i = i0 + e;  // index into the centre-padded clip
+    v[e] = 0.f;
     if (i < padded_len) {
       int64_t j = i - pad;
       if (j < 0) j = (pad_mode == NNAB_PAD_REFLECT) ? -j : -1;
       else if (j >= L) j = (pad_mode == NNAB_PAD_REFLECT) ? 2 * (L - 1) - j : -1;
-      if (j >= 0 && j < L) v = __ldg(xb + j);
+      if (j >= 0 && j < L) v[e] = ldg_sample(xb + j);
     }
-    split_bf16(v, hi[e], lo[e]);
   }
+}
+
+// One thread = 8 consecutive samples of one clip's slot region (16-byte stores).  hi_only: the lo
+// plane is left alone (bf16 input: it would be all zeros, and the two-term kernels never read it).
+template <typename T>
+__global__ void __launch_bounds__(256) pad_split_kernel(
+    const T* __restrict__ x, int64_t L, int64_t x_pitch, int pad, int pad_mode, int shift,
+    int64_t clip_pitch, int64_t plane_stride, __nv_bfloat16* __restrict__ planes, int hi_only) {
+  const int64_t b = blockIdx.y;
+  const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 8;
+  if (i0 >= clip_pitch) return;
+  const T* __restrict__ xb = x + b * x_pitch;
+  float v[8];
+  fetch8_padded(xb, L, i0 + shift, pad, pad_mode, v);
+  __align__(16) __nv_bfloat16 hi[8];
+  __align__(16) __nv_bfloat16 lo[8];
+#pragma unroll
+  for (int e = 0; e < 8; ++e) split_bf16(v[e], hi[e], lo[e]);
   const int64_t o = b * clip_pitch + i0;
   *reinterpret_cast<uint4*>(planes + o) = *reinterpret_cast<const uint4*>(hi);
-  *reinterpret_cast<uint4*>(planes + plane_stride + o) = *reinterpret_cast<const uint4*>(lo);
+  if (!hi_only)
+    *reinterpret_cast<uint4*>(planes + plane_stride + o) = *reinterpret_cast<const uint4*>(lo);
 }
 
 // Two differently padded split copies of the same batch in one pass over x (level 0 of
 // the CQT pyramid: reflect-padded copy for the octave CQT + zero-margin copy for the FIR).
+template <typename T>
 __global__ void __launch_bounds__(256) pad_split2_kernel(
-    const float* __restrict__ x, int64_t L, int64_t x_pitch,
+    const T* __restrict__ x, int64_t L, int64_t x_pitch,
     int pad_a, int mode_a, int64_t pitch_a, int64_t plane_a, __nv_bfloat16* __restrict__ pa,
     int pad_b, int mode_b, int64_t pitch_b, int64_t plane_b, __nv_bfloat16* __restrict__ pb) {
   const int64_t b = blockIdx.y;
   const int64_t i0 = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) * 8;
-  const float* __restrict__ xb = x + b * x_pitch;
+  const T* __restrict__ xb = x + b * x_pitch;
 #pragma unroll
   for (int which = 0; which < 2; ++which) {
     const int pad = which ? pad_b : pad_a;
@@ -147,25 +168,41 @@ __global__ void __launch_bounds__(256) pad_split2_kernel(
     const int64_t plane = which ? plane_b : plane_a;
     __nv_bfloat16* __restrict__ dst = which ? pb : pa;
     if (i0 >= pitch) continue;
-    const int64_t padded_len = L + 2 * (int64_t)pad;
+    float v[8];
+    fetch8_padded(xb, L, i0, pad, mode, v);
     __align__(16) __nv_bfloat16 hi[8];
     __align__(16) __nv_bfloat16 lo[8];
 #pragma unroll
-    for (int e = 0; e < 8; ++e) {
-      const int64_t i = i0 + e;
-      float v = 0.f;
-      if (i < padded_len) {
-        int64_t j = i - pad;
-        if (j < 0) j = (mode == NNAB_PAD_REFLECT) ? -j : -1;
-        else if (j >= L) j = (mode == NNAB_PAD_REFLECT) ? 2 * (L - 1) - j : -1;
-        if (j >= 0 && j < L) v = __ldg(xb + j);
-      }
-      split_bf16(v, hi[e], lo[e]);
-    }
+    for (int e = 0; e < 8; ++e) split_bf16(v[e], hi[e], lo[e]);
     const int64_t o = b * pitch + i0;
     *reinterpret_cast<uint4*>(dst + o) = *reinterpret_cast<const uint4*>(hi);
     *reinterpret_cast<uint4*>(dst + plane + o) = *reinterpret_cast<const uint4*>(lo);
   }
+}
+
+// pad_split_kernel launch for the element type of x
+static int launch_pad_split(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int pad,
+                            int pad_mode, int shift, int64_t clip_pitch, int64_t plane_stride,
+                            __nv_bfloat16* planes, bool hi_only, cudaStream_t stream) {
+  if (hi_only && x_dtype != NNAB_DTYPE_BF16) return NNAB_EINVAL;
+  dim3 grid((unsigned)ceil_div64(clip_pitch, 256 * 8), (unsigned)B);
+  switch (x_dtype) {
+    case NNAB_DTYPE_F32:
+      pad_split_kernel<<<grid, 256, 0, stream>>>((const float*)x, L, x_pitch, pad, pad_mode, shift,
+                                                 clip_pitch, plane_stride, planes, 0);
+      break;
+    case NNAB_DTYPE_BF16:
+      pad_split_kernel<<<grid, 256, 0, stream>>>((const __nv_bfloat16*)x, L, x_pitch, pad, pad_mode,
+                                                 shift, clip_pitch, plane_stride, planes, hi_only ? 1 : 0);
+      break;
+    case NNAB_DTYPE_F16:
+      pad_split_kernel<<<grid, 256, 0, stream>>>((const __half*)x, L, x_pitch, pad, pad_mode, shift,
+                                                 clip_pitch, plane_stride, planes, 0);
+      break;
+    default: return NNAB_EINVAL;
+  }
+  NNAB_LAUNCH_CHECK();
+  return NNAB_OK;
 }
 
 // packed[plane][tile*bn + part*bn/2 + j][k]; part 1 rows are NEGATED im rows.
@@ -272,29 +309,27 @@ void tc_split_geometry(int64_t B, int64_t L, int K, int hop, int pad, int64_t* t
   if (hop_eff) *hop_eff = hop * num_phases(hop);
 }
 
-static int zero_tail(__nv_bfloat16* planes, const SplitGeom& g, int hop_eff, cudaStream_t stream) {
+static int zero_tail(__nv_bfloat16* planes, const SplitGeom& g, int hop_eff, cudaStream_t stream,
+                     bool hi_only = false) {
   const int64_t tail = g.plane_stride - g.nv * hop_eff;
-  for (int pl = 0; pl < 2; ++pl)
+  for (int pl = 0; pl < (hi_only ? 1 : 2); ++pl)
     NNAB_CUDA_TRY(cudaMemsetAsync(planes + pl * g.plane_stride + g.nv * hop_eff, 0,
                                   (size_t)tail * sizeof(__nv_bfloat16), stream));
   return NNAB_OK;
 }
 
-// phase-0 pad + split of an fp32 batch into caller-managed planes
-int tc_pad_split(const float* x, int64_t B, int64_t L, int64_t x_pitch, int K, int hop, int pad,
-                 int pad_mode, void* planes_v, cudaStream_t stream) {
+// phase-0 pad + split of a batch into caller-managed planes
+int tc_pad_split(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int K, int hop,
+                 int pad, int pad_mode, void* planes_v, cudaStream_t stream, bool hi_only) {
   if (B > 65535) return NNAB_EUNSUPPORTED;
   const SplitGeom g = split_geom(B, L, K, hop, pad);
   const int hop_eff = hop * num_phases(hop);
   __nv_bfloat16* planes = (__nv_bfloat16*)planes_v;
-  int rc = zero_tail(planes, g, hop_eff, stream);
+  int rc = zero_tail(planes, g, hop_eff, stream, hi_only);
   if (rc) return rc;
   const int64_t clip_pitch = g.t_slots * hop_eff;
-  dim3 grid((unsigned)ceil_div64(clip_pitch, 256 * 8), (unsigned)B);
-  pad_split_kernel<<<grid, 256, 0, stream>>>(x, L, x_pitch, pad, pad_mode, 0, clip_pitch,
-                                             g.plane_stride, planes);
-  NNAB_LAUNCH_CHECK();
-  return NNAB_OK;
+  return launch_pad_split(x, x_dtype, B, L, x_pitch, pad, pad_mode, 0, clip_pitch, g.plane_stride,
+                          planes, hi_only, stream);
 }
 
 __global__ void zero_margins_kernel(__nv_bfloat16* __restrict__ planes, int64_t plane_stride,
@@ -303,8 +338,9 @@ __global__ void zero_margins_kernel(__nv_bfloat16* __restrict__ planes, int64_t 
 // pad + split into caller-defined geometry (clip pitch / plane stride in elements).  pad_split_kernel
 // writes the whole [0, clip_pitch) slot of every clip (zeros past the padded signal); the tail
 // [B * clip_pitch, plane_stride) is zeroed here.
-int tc_pad_split_ex(const float* x, int64_t B, int64_t L, int64_t x_pitch, int pad, int pad_mode,
-                    int64_t clip_pitch, int64_t plane_stride, void* planes_v, cudaStream_t stream) {
+int tc_pad_split_ex(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch, int pad,
+                    int pad_mode, int64_t clip_pitch, int64_t plane_stride, void* planes_v,
+                    cudaStream_t stream) {
   if (B > 65535) return NNAB_EUNSUPPORTED;
   if (clip_pitch % 8 != 0 || plane_stride < B * clip_pitch) return NNAB_EINVAL;
   __nv_bfloat16* planes = (__nv_bfloat16*)planes_v;
@@ -312,11 +348,8 @@ int tc_pad_split_ex(const float* x, int64_t B, int64_t L, int64_t x_pitch, int p
   for (int pl = 0; pl < 2 && tail > 0; ++pl)
     NNAB_CUDA_TRY(cudaMemsetAsync(planes + pl * plane_stride + B * clip_pitch, 0,
                                   (size_t)tail * sizeof(__nv_bfloat16), stream));
-  dim3 grid((unsigned)ceil_div64(clip_pitch, 256 * 8), (unsigned)B);
-  pad_split_kernel<<<grid, 256, 0, stream>>>(x, L, x_pitch, pad, pad_mode, 0, clip_pitch, plane_stride,
-                                             planes);
-  NNAB_LAUNCH_CHECK();
-  return NNAB_OK;
+  return launch_pad_split(x, x_dtype, B, L, x_pitch, pad, pad_mode, 0, clip_pitch, plane_stride, planes,
+                          false, stream);
 }
 
 // zero [keep_hi, clip_pitch) and [0, keep_lo) of every clip slot (both planes) + the tail of the planes
@@ -340,7 +373,7 @@ int tc_zero_slots(void* planes_v, int64_t B, int64_t clip_pitch, int64_t plane_s
   return NNAB_OK;
 }
 
-int tc_pad_split2(const float* x, int64_t B, int64_t L, int64_t x_pitch,
+int tc_pad_split2(const void* x, int x_dtype, int64_t B, int64_t L, int64_t x_pitch,
                   int K_a, int hop_a, int pad_a, int mode_a, void* planes_a,
                   int K_b, int hop_b, int pad_b, int mode_b, void* planes_b, cudaStream_t stream) {
   if (B > 65535) return NNAB_EUNSUPPORTED;
@@ -353,10 +386,26 @@ int tc_pad_split2(const float* x, int64_t B, int64_t L, int64_t x_pitch,
   const int64_t pitch_a = ga.t_slots * he_a, pitch_b = gb.t_slots * he_b;
   const int64_t pmax = pitch_a > pitch_b ? pitch_a : pitch_b;
   dim3 grid((unsigned)ceil_div64(pmax, 256 * 8), (unsigned)B);
-  pad_split2_kernel<<<grid, 256, 0, stream>>>(x, L, x_pitch, pad_a, mode_a, pitch_a,
-                                              ga.plane_stride, (__nv_bfloat16*)planes_a, pad_b,
-                                              mode_b, pitch_b, gb.plane_stride,
-                                              (__nv_bfloat16*)planes_b);
+  __nv_bfloat16* pa = (__nv_bfloat16*)planes_a;
+  __nv_bfloat16* pb = (__nv_bfloat16*)planes_b;
+  switch (x_dtype) {
+    case NNAB_DTYPE_F32:
+      pad_split2_kernel<<<grid, 256, 0, stream>>>((const float*)x, L, x_pitch, pad_a, mode_a, pitch_a,
+                                                  ga.plane_stride, pa, pad_b, mode_b, pitch_b,
+                                                  gb.plane_stride, pb);
+      break;
+    case NNAB_DTYPE_BF16:
+      pad_split2_kernel<<<grid, 256, 0, stream>>>((const __nv_bfloat16*)x, L, x_pitch, pad_a, mode_a,
+                                                  pitch_a, ga.plane_stride, pa, pad_b, mode_b, pitch_b,
+                                                  gb.plane_stride, pb);
+      break;
+    case NNAB_DTYPE_F16:
+      pad_split2_kernel<<<grid, 256, 0, stream>>>((const __half*)x, L, x_pitch, pad_a, mode_a, pitch_a,
+                                                  ga.plane_stride, pa, pad_b, mode_b, pitch_b,
+                                                  gb.plane_stride, pb);
+      break;
+    default: return NNAB_EINVAL;
+  }
   NNAB_LAUNCH_CHECK();
   return NNAB_OK;
 }
@@ -697,6 +746,7 @@ struct TcParams {
   int t_mul, t_add;  // output frame index = t * t_mul + t_add (frame phases)
   int k_splits;      // >1: every (m, n) tile is cut into k_splits K-chunks (FMT_RAW epilogue)
   int split4;        // EXPERIMENTAL (NNAB_SPLIT4=1): add the x_lo * w_lo term (4 MMAs per K16 step)
+  int two_term;      // bf16 input: the A lo plane is zero -- neither loaded nor multiplied
   int64_t nv, t_slots, T;  // T = valid frames of this phase
   int kb_begin[TC_MAX_N_TILES];
   int kb_end[TC_MAX_N_TILES];
@@ -937,7 +987,7 @@ framed_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t sb = base + stage * S::STAGE_BYTES;
-          mbar_expect_tx(full_bar(stage), 2 * S::A_BYTES + 2 * b_tile_bytes);
+          mbar_expect_tx(full_bar(stage), (p.two_term ? 1 : 2) * S::A_BYTES + 2 * b_tile_bytes);
           const int k0 = kb * BK;
           int c0 = k0, c1 = m0;
           if (p.rows_mode) {
@@ -945,7 +995,7 @@ framed_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             c0 = k0 - (k0 / p.hop) * p.hop;
           }
           tma_load_3d(sb, &tm_a, full_bar(stage), c0, c1, 0);
-          tma_load_3d(sb + S::A_BYTES, &tm_a, full_bar(stage), c0, c1, 1);
+          if (!p.two_term) tma_load_3d(sb + S::A_BYTES, &tm_a, full_bar(stage), c0, c1, 1);
           tma_load_3d(sb + 2 * S::A_BYTES, &tm_b, full_bar(stage), k0, n0, 0);
           tma_load_3d(sb + 2 * S::A_BYTES + S::B_BYTES, &tm_b, full_bar(stage), k0, n0, 1);
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
@@ -981,8 +1031,11 @@ framed_tc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant
             const uint64_t a_lo = make_smem_desc<BK>(sb + S::A_BYTES + koff);
             const uint64_t b_hi = make_smem_desc<BK>(sb + 2 * S::A_BYTES + koff);
             const uint64_t b_lo = make_smem_desc<BK>(sb + 2 * S::A_BYTES + S::B_BYTES + koff);
-            umma_bf16(d_tmem, a_lo, b_hi, idesc, accumulate);
-            umma_bf16(d_tmem, a_hi, b_lo, idesc, 1u);
+            if (!p.two_term) {
+              umma_bf16(d_tmem, a_lo, b_hi, idesc, accumulate);
+              accumulate = 1u;
+            }
+            umma_bf16(d_tmem, a_hi, b_lo, idesc, accumulate);
             umma_bf16(d_tmem, a_hi, b_hi, idesc, 1u);
             accumulate = 1u;
           }
@@ -1106,7 +1159,7 @@ framed_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
         for (int kb = kb0; kb < kb1; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t sb = base + stage * S::STAGE_BYTES;
-          mbar_expect_tx_remote(full_bar(stage), 0, 2 * S::A_BYTES + 2 * b_half_bytes);
+          mbar_expect_tx_remote(full_bar(stage), 0, (p.two_term ? 1 : 2) * S::A_BYTES + 2 * b_half_bytes);
           const int k0 = kb * BK;
           int c0 = k0, c1 = m0;
           if (p.rows_mode) {
@@ -1114,7 +1167,7 @@ framed_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             c0 = k0 - (k0 / p.hop) * p.hop;
           }
           tma_load_3d_2sm(sb, &tm_a, full_bar(stage), c0, c1, 0);
-          tma_load_3d_2sm(sb + S::A_BYTES, &tm_a, full_bar(stage), c0, c1, 1);
+          if (!p.two_term) tma_load_3d_2sm(sb + S::A_BYTES, &tm_a, full_bar(stage), c0, c1, 1);
           tma_load_3d_2sm(sb + 2 * S::A_BYTES, &tm_b, full_bar(stage), k0, n0, 0);
           tma_load_3d_2sm(sb + 2 * S::A_BYTES + S::B_BYTES, &tm_b, full_bar(stage), k0, n0, 1);
           if (++stage == STAGES) { stage = 0; phase ^= 1u; }
@@ -1149,12 +1202,15 @@ framed_tc2_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             const uint64_t a_lo = make_smem_desc<BK>(sb + S::A_BYTES + koff);
             const uint64_t b_hi = make_smem_desc<BK>(sb + 2 * S::A_BYTES + koff);
             const uint64_t b_lo = make_smem_desc<BK>(sb + 2 * S::A_BYTES + S::B_BYTES + koff);
-            if (p.split4) {  // smallest term first: fp32-like accuracy for the training forward
-              umma_bf16_2sm(d_tmem, a_lo, b_lo, idesc, accumulate);
+            if (!p.two_term) {
+              if (p.split4) {  // smallest term first: fp32-like accuracy for the training forward
+                umma_bf16_2sm(d_tmem, a_lo, b_lo, idesc, accumulate);
+                accumulate = 1u;
+              }
+              umma_bf16_2sm(d_tmem, a_lo, b_hi, idesc, accumulate);
               accumulate = 1u;
             }
-            umma_bf16_2sm(d_tmem, a_lo, b_hi, idesc, accumulate);
-            umma_bf16_2sm(d_tmem, a_hi, b_lo, idesc, 1u);
+            umma_bf16_2sm(d_tmem, a_hi, b_lo, idesc, accumulate);
             umma_bf16_2sm(d_tmem, a_hi, b_hi, idesc, 1u);
             accumulate = 1u;
           }
@@ -1344,14 +1400,15 @@ framed_tc2v_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
           const int rows = 8 * (int)plan.groups[i];  // basis rows this CTA stages
           mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t sb = base + stage * S::STAGE_BYTES;
-          mbar_expect_tx_remote(full_bar(stage), 0, 2 * S::A_BYTES + 2 * (uint32_t)rows * BK * 2);
+          mbar_expect_tx_remote(full_bar(stage), 0,
+                                (p.two_term ? 1 : 2) * S::A_BYTES + 2 * (uint32_t)rows * BK * 2);
           int c0 = k0, c1 = m0;
           if (p.rows_mode) {
             c1 = m0 + k0 / p.hop;
             c0 = k0 - (k0 / p.hop) * p.hop;
           }
           tma_load_3d_2sm(sb, &tm_a, full_bar(stage), c0, c1, 0);
-          tma_load_3d_2sm(sb + S::A_BYTES, &tm_a, full_bar(stage), c0, c1, 1);
+          if (!p.two_term) tma_load_3d_2sm(sb + S::A_BYTES, &tm_a, full_bar(stage), c0, c1, 1);
           const int row0 = (int)cta * rows;
           const uint32_t bh = sb + 2 * S::A_BYTES, bl = bh + S::B_BYTES;
           int r = 0;
@@ -1392,8 +1449,11 @@ framed_tc2v_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
             const uint64_t a_lo = make_smem_desc<BK>(sb + S::A_BYTES + koff);
             const uint64_t b_hi = make_smem_desc<BK>(sb + 2 * S::A_BYTES + koff);
             const uint64_t b_lo = make_smem_desc<BK>(sb + 2 * S::A_BYTES + S::B_BYTES + koff);
-            umma_bf16_2sm(d_tmem, a_lo, b_hi, idesc, accumulate);
-            umma_bf16_2sm(d_tmem, a_hi, b_lo, idesc, 1u);
+            if (!p.two_term) {
+              umma_bf16_2sm(d_tmem, a_lo, b_hi, idesc, accumulate);
+              accumulate = 1u;
+            }
+            umma_bf16_2sm(d_tmem, a_hi, b_lo, idesc, accumulate);
             umma_bf16_2sm(d_tmem, a_hi, b_hi, idesc, 1u);
             accumulate = 1u;
           }
@@ -1775,13 +1835,13 @@ static int launch_framed_tc_varn(const FramedProblem& q, const void* packed, voi
   const int rows_w = 16 * ((q.F + 7) / 8);
   __nv_bfloat16* planes =
       reinterpret_cast<__nv_bfloat16*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-  int rc = zero_tail(planes, g, q.hop, stream);
+  const bool two = two_term(q);
+  int rc = zero_tail(planes, g, q.hop, stream, two);
   if (rc) return rc;
   const int64_t clip_pitch = g.t_slots * q.hop;
-  dim3 pgrid((unsigned)ceil_div64(clip_pitch, 256 * 8), (unsigned)q.B);
-  pad_split_kernel<<<pgrid, 256, 0, stream>>>(q.x, q.L, q.x_pitch, q.pad, q.pad_mode, 0, clip_pitch,
-                                              g.plane_stride, planes);
-  NNAB_LAUNCH_CHECK();
+  if ((rc = launch_pad_split(q.x, q.x_dtype, q.B, q.L, q.x_pitch, q.pad, q.pad_mode, 0, clip_pitch,
+                             g.plane_stride, planes, two, stream)))
+    return rc;
 
   // split-K only with the caller's raw scratch (long kernels): <= 64 K blocks per accumulator
   VarNPlan plan;
@@ -1829,6 +1889,7 @@ static int launch_framed_tc_varn(const FramedProblem& q, const void* packed, voi
   prm.t_add = 0;
   prm.T = q.T;
   prm.k_splits = plan.n_chunks;
+  prm.two_term = two ? 1 : 0;
   prm.epi.scale = q.scale; prm.epi.scale_all = q.scale_all; prm.epi.fmt = q.fmt;
   prm.epi.eps = q.eps; prm.epi.power = q.power; prm.epi.out = q.out; prm.epi.T = q.T;
   prm.epi.out_bins = q.out_bins; prm.epi.bin_offset = q.bin_offset; prm.epi.F = q.F;
@@ -1853,7 +1914,7 @@ static int launch_framed_tc_varn(const FramedProblem& q, const void* packed, voi
   {
     double cols = 0.0;
     for (int i = 0; i < plan.n_blocks; ++i) cols += 16.0 * plan.groups[i] * 64.0;
-    add_exec_flops(3.0 * 2.0 * (double)prm.num_m_tiles * (2 * TC_BM) * cols);
+    add_exec_flops((two ? 2.0 : 3.0) * 2.0 * (double)prm.num_m_tiles * (2 * TC_BM) * cols);
   }
   switch (prm.epi.fmt) {
     case NNAB_FMT_MAGNITUDE: rc = launch_tc2v_fmt<0>(ma, mb8, mb32, prm, plan, n_pairs, stream); break;
@@ -1914,8 +1975,9 @@ int launch_framed_tc(const FramedProblem& q, const void* packed, void* workspace
 
   // K overhang rows past the last clip must be finite zeros (the basis is zero-padded there)
   const int64_t clip_pitch = g.t_slots * hop_eff;
+  const bool two = two_term(q);
   if (q.presplit == nullptr) {
-    const int zrc = zero_tail(planes, g, hop_eff, stream);
+    const int zrc = zero_tail(planes, g, hop_eff, stream, two);
     if (zrc) return zrc;
   }
 
@@ -1960,6 +2022,7 @@ int launch_framed_tc(const FramedProblem& q, const void* packed, void* workspace
     const char* e4 = getenv("NNAB_SPLIT4");
     prm.split4 = (e4 != nullptr && atoi(e4) == 1) ? 1 : 0;  // CTA-pair kernel only
   }
+  prm.two_term = two ? 1 : 0;
   const int nkb = kpad / bk;
   const int half = bn / 2;
   for (int tl = 0; tl < n_tiles; ++tl) {
@@ -2037,17 +2100,16 @@ int launch_framed_tc(const FramedProblem& q, const void* packed, void* workspace
     if (ph >= q.T) break;
     prm.t_add = ph;
     prm.T = (q.T - ph + n_ph - 1) / n_ph;  // frames t = ph, ph + n_ph, ... < T
-    if (q.presplit == nullptr) {
-      dim3 grid((unsigned)ceil_div64(clip_pitch, 256 * 8), (unsigned)q.B);
-      pad_split_kernel<<<grid, 256, 0, stream>>>(q.x, q.L, q.x_pitch, q.pad, q.pad_mode,
-                                                 ph * q.hop, clip_pitch, g.plane_stride, planes);
-      NNAB_LAUNCH_CHECK();
-    }
+    if (q.presplit == nullptr &&
+        (rc = launch_pad_split(q.x, q.x_dtype, q.B, q.L, q.x_pitch, q.pad, q.pad_mode, ph * q.hop,
+                               clip_pitch, g.plane_stride, planes, two, stream)))
+      return rc;
     {
       const int mrows = (cta_group == 2 ? 2 : 1) * TC_BM;
       double kcols = 0.0;  // sum over N tiles of (k-blocks executed) x bk x bn
       for (int tl = 0; tl < n_tiles; ++tl) kcols += (double)(prm.kb_end[tl] - prm.kb_begin[tl]) * bk * bn;
-      add_exec_flops((prm.split4 && cta_group == 2 ? 4.0 : 3.0) * 2.0 *
+      const double terms = two ? 2.0 : (prm.split4 && cta_group == 2 ? 4.0 : 3.0);
+      add_exec_flops(terms * 2.0 *
                      (double)ceil_div64(g.nv, mrows) * mrows * kcols);
     }
     if (cta_group == 2) {

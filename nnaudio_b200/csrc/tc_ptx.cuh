@@ -230,6 +230,20 @@ __device__ __forceinline__ void umma_kblock_split3(uint32_t d_tmem, uint32_t a_h
   }
 }
 
+// the same K block for a bf16 A operand (zero lo plane): A_hi x (B_hi, B_lo) only
+__device__ __forceinline__ void umma_kblock_split2(uint32_t d_tmem, uint32_t a_hi_lo, uint32_t b_hi_lo,
+                                                   uint32_t b_lo_lo, uint32_t hi, uint32_t idesc,
+                                                   bool first_accumulates) {
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    const uint64_t a_hi = desc64(a_hi_lo + 2u * k, hi);
+    const uint64_t b_hi = desc64(b_hi_lo + 2u * k, hi), b_lo = desc64(b_lo_lo + 2u * k, hi);
+    if (k == 0 && !first_accumulates) umma_bf16_2sm_i<false>(d_tmem, a_hi, b_lo, idesc);
+    else umma_bf16_2sm_i<true>(d_tmem, a_hi, b_lo, idesc);
+    umma_bf16_2sm_i<true>(d_tmem, a_hi, b_hi, idesc);
+  }
+}
+
 __device__ __forceinline__ void tma_load_4d_2sm(uint32_t dst, const CUtensorMap* map, uint32_t bar,
                                                 int c0, int c1, int c2, int c3) {
   asm volatile(

@@ -50,6 +50,7 @@ struct TcbParams {
   int num_n_tiles;
   int nb;            // packed bins per N tile (MMA N = 2 nb)
   int kb_n;          // hop / 64
+  int two_term;      // bf16 input: the A lo plane is zero -- neither loaded nor multiplied
   int64_t nv, t_slots, T;
   EpiParams epi;
 };
@@ -441,14 +442,15 @@ framed_tcb_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
         for (int kb = 0; kb < p.kb_n; ++kb) {
           mbar_wait(empty_bar(stage), phase ^ 1u);
           const uint32_t sb = base + stage * S::STAGE_BYTES;
-          mbar_expect_tx_remote(full_bar(stage), 0, 2 * S::A_BYTES + 2 * b_bytes);
+          mbar_expect_tx_remote(full_bar(stage), 0, (p.two_term ? 1 : 2) * S::A_BYTES + 2 * b_bytes);
           const int k0 = kb * BK;
 #pragma unroll
           for (int q = 0; q < 4; ++q) {  // 32-row boxes, row origins FW apart
             tma_load_3d_2sm(sb + (uint32_t)q * 32u * BK * 2u, &tm_a, full_bar(stage), k0,
                             m0 + q * FW, 0);
-            tma_load_3d_2sm(sb + S::A_BYTES + (uint32_t)q * 32u * BK * 2u, &tm_a, full_bar(stage), k0,
-                            m0 + q * FW, 1);
+            if (!p.two_term)
+              tma_load_3d_2sm(sb + S::A_BYTES + (uint32_t)q * 32u * BK * 2u, &tm_a, full_bar(stage), k0,
+                              m0 + q * FW, 1);
           }
           tma_load_3d_2sm(sb + 2 * S::A_BYTES, &tm_b, full_bar(stage), k0, n0, (int)cta);
           tma_load_3d_2sm(sb + 2 * S::A_BYTES + S::B_BYTES, &tm_b, full_bar(stage), k0, n0,
@@ -482,8 +484,11 @@ framed_tcb_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constan
             const uint64_t a_lo = make_smem_desc<BK>(sb + S::A_BYTES + koff);
             const uint64_t b_hi = make_smem_desc<BK>(sb + 2 * S::A_BYTES + koff);
             const uint64_t b_lo = make_smem_desc<BK>(sb + 2 * S::A_BYTES + S::B_BYTES + koff);
-            umma_bf16_2sm(d_tmem, a_lo, b_hi, idesc, accumulate);
-            umma_bf16_2sm(d_tmem, a_hi, b_lo, idesc, 1u);
+            if (!p.two_term) {
+              umma_bf16_2sm(d_tmem, a_lo, b_hi, idesc, accumulate);
+              accumulate = 1u;
+            }
+            umma_bf16_2sm(d_tmem, a_hi, b_lo, idesc, accumulate);
             umma_bf16_2sm(d_tmem, a_hi, b_hi, idesc, 1u);
             accumulate = 1u;
           }
@@ -609,7 +614,9 @@ int launch_framed_tc_block(const FramedProblem& q, const void* packed, void* wor
   const SplitGeom g = split_geom(q.B, q.L, q.K, q.hop, q.pad);
   __nv_bfloat16* planes =
       reinterpret_cast<__nv_bfloat16*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-  int rc = tc_pad_split(q.x, q.B, q.L, q.x_pitch, q.K, q.hop, q.pad, q.pad_mode, planes, stream);
+  const bool two = two_term(q);
+  int rc = tc_pad_split(q.x, q.x_dtype, q.B, q.L, q.x_pitch, q.K, q.hop, q.pad, q.pad_mode, planes, stream,
+                        two);
   if (rc) return rc;
 
   int dev = 0, sms = 148;
@@ -649,6 +656,7 @@ int launch_framed_tc_block(const FramedProblem& q, const void* packed, void* wor
   prm.num_n_tiles = n_tiles;
   prm.nb = nb;
   prm.kb_n = q.hop / 64;
+  prm.two_term = two ? 1 : 0;
   prm.nv = g.nv;
   prm.t_slots = g.t_slots;
   prm.T = q.T;
@@ -662,7 +670,7 @@ int launch_framed_tc_block(const FramedProblem& q, const void* packed, void* wor
   if (q.fmt == FMT_PLANES && (int64_t)n_tiles * nb > q.planes_pitch) return NNAB_EINVAL;
   const int64_t ptiles = (int64_t)prm.num_m_pairs * n_tiles;
   const int n_pairs = (int)(ptiles < sms / 2 ? ptiles : sms / 2);
-  add_exec_flops(3.0 * 2.0 * (double)ptiles * (2 * TC_BM) * (2 * nb) * q.hop);
+  add_exec_flops((two ? 2.0 : 3.0) * 2.0 * (double)ptiles * (2 * TC_BM) * (2 * nb) * q.hop);
   return R == 4 ? launch_tcb<4>(q.fmt, ma, mb, prm, n_pairs, stream)
                 : launch_tcb<2>(q.fmt, ma, mb, prm, n_pairs, stream);
 }

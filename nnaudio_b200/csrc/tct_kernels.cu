@@ -60,6 +60,7 @@ struct TallPlan {
 struct TctParams {
   int num_m_tiles;                // 256-frame pair tiles (per frame phase)
   int n_phases;                   // frames t = s * n_phases + p: phase p reads the planes shifted by p * hop
+  int two_term;                   // bf16 input: the A lo plane is zero -- neither loaded nor multiplied
   int64_t nv, t_slots, T;         // per phase: virtual frames, frames per clip slot; T = frames of the output
   EpiParams epi;
   float* sk_scratch;              // balanced schedule only: partial sums of the tiles two pairs share
@@ -212,9 +213,9 @@ framed_tc2t_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
           // ---- the column's tall A block: rows m0 + r_min .. + a_rows, columns [64 c, 64 c + 64)
           mbar_wait(a_empty(abuf), aphase ^ 1u);
           const uint32_t ab = base + (uint32_t)abuf * S::A_BUF;
-          mbar_expect_tx_remote(a_full(abuf), 0, 2u * (uint32_t)plan.a_rows * BK * 2u);
+          mbar_expect_tx_remote(a_full(abuf), 0, (p.two_term ? 1u : 2u) * (uint32_t)plan.a_rows * BK * 2u);
           tma_load_4d_2sm(ab, &tm_a, a_full(abuf), c * BK, ph, m0 + r_min, 0);
-          tma_load_4d_2sm(ab + S::A_PLANE, &tm_a, a_full(abuf), c * BK, ph, m0 + r_min, 1);
+          if (!p.two_term) tma_load_4d_2sm(ab + S::A_PLANE, &tm_a, a_full(abuf), c * BK, ph, m0 + r_min, 1);
           if (++abuf == 2) { abuf = 0; aphase ^= 1u; }
           // ---- the basis rows of every K block of this column
           for (int i = 0; i < r_cnt; ++i) {
@@ -261,9 +262,13 @@ framed_tc2t_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_consta
             tcgen05_fence_after();
             const uint32_t bh = base + S::B_OFFSET + (uint32_t)stage * S::B_STAGE;
             const uint32_t a_row = (uint32_t)plan.shift[plan.col_off[ci] + i] * (BK * 2);  // r rows down
-            umma_kblock_split3(d_tmem, smem_desc_lo<BK>(ab + a_row), smem_desc_lo<BK>(ab + S::A_PLANE + a_row),
-                               smem_desc_lo<BK>(bh), smem_desc_lo<BK>(bh + S::B_PLANE), smem_desc_hi<BK>(),
-                               idesc, accumulate != 0);
+            if (p.two_term)
+              umma_kblock_split2(d_tmem, smem_desc_lo<BK>(ab + a_row), smem_desc_lo<BK>(bh),
+                                 smem_desc_lo<BK>(bh + S::B_PLANE), smem_desc_hi<BK>(), idesc, accumulate != 0);
+            else
+              umma_kblock_split3(d_tmem, smem_desc_lo<BK>(ab + a_row), smem_desc_lo<BK>(ab + S::A_PLANE + a_row),
+                                 smem_desc_lo<BK>(bh), smem_desc_lo<BK>(bh + S::B_PLANE), smem_desc_hi<BK>(),
+                                 idesc, accumulate != 0);
             accumulate = 1u;
             umma_commit_2sm(b_empty(stage));
             if (++stage == BS) { stage = 0; phase ^= 1u; }
@@ -526,7 +531,8 @@ int launch_framed_tc_tall(const FramedProblem& q, const void* packed, void* work
     if (workspace == nullptr || ws_bytes < need) return NNAB_EWORKSPACE;
     const SplitGeom g = split_geom(q.B, q.L, q.K, q.hop, q.pad);
     planes = reinterpret_cast<__nv_bfloat16*>(((uintptr_t)workspace + 255) & ~(uintptr_t)255);
-    rc = tc_pad_split(q.x, q.B, q.L, q.x_pitch, q.K, q.hop, q.pad, q.pad_mode, planes, stream);
+    rc = tc_pad_split(q.x, q.x_dtype, q.B, q.L, q.x_pitch, q.K, q.hop, q.pad, q.pad_mode, planes, stream,
+                      two_term(q));
     if (rc) return rc;
     t_slots = g.t_slots;
     plane_stride = g.plane_stride;
@@ -562,6 +568,7 @@ int launch_framed_tc_tall(const FramedProblem& q, const void* packed, void* work
   prm.sk_flags = nullptr;
   prm.num_m_tiles = (int)ceil_div64(nv, 2 * TC_BM);
   prm.n_phases = P;
+  prm.two_term = two_term(q) ? 1 : 0;
   prm.nv = nv;
   prm.t_slots = t_slots;
   prm.T = q.T;
@@ -577,7 +584,7 @@ int launch_framed_tc_tall(const FramedProblem& q, const void* packed, void* work
   {
     double cols = 0.0;
     for (int kb = 0; kb < TCT_MAX_KB; ++kb) cols += 16.0 * plan.groups[kb] * 64.0;
-    add_exec_flops(3.0 * 2.0 * (double)tiles * (2 * TC_BM) * cols);
+    add_exec_flops((prm.two_term ? 2.0 : 3.0) * 2.0 * (double)tiles * (2 * TC_BM) * cols);
   }
   // Balanced schedule (TallSched<true>): only when the static one leaves a ragged last round, and the
   // split-K scratch of this problem (long kernels: attach_splitk_scratch) can hold one slot per pair.

@@ -60,7 +60,9 @@ class FramedComplexFn(torch.autograd.Function):
     forward = the fused kernel; backward = ``nnab_framed_backward_input`` (GEMM with the
     transposed basis + overlap-add + padding adjoint) for ``x`` and
     ``nnab_framed_backward_weight`` (split-K GEMM over all frames) for the bases
-    (the reference gets both from autograd through conv1d, stft.py:290-293)."""
+    (the reference gets both from autograd through conv1d, stft.py:290-293).  A bf16 / fp16 ``x``
+    runs the forward kernel on the 16-bit samples; its gradient is the fp32 one cast to ``x.dtype``,
+    and the weight gradient reads ``x.float()``."""
 
     @staticmethod
     def forward(ctx, x, w_re, w_im, fwd, bwd_x, bwd_w):
@@ -77,9 +79,9 @@ class FramedComplexFn(torch.autograd.Function):
         g = g.contiguous()
         dx = dre = dim = None
         if ctx.needs_input_grad[0]:
-            dx = ctx.bwd_x(g, ctx.in_shape[-1]).reshape(ctx.in_shape)
+            dx = ctx.bwd_x(g, ctx.in_shape[-1]).reshape(ctx.in_shape).to(x.dtype)
         if ctx.needs_input_grad[1] or ctx.needs_input_grad[2]:
-            dre, dim = ctx.bwd_w(g, x)
+            dre, dim = ctx.bwd_w(g, x.float())
             dre, dim = dre.reshape(ctx.w_shape), dim.reshape(ctx.w_shape)
         return dx, dre, dim, None, None, None
 

@@ -234,7 +234,7 @@ class _CFPBase(nn.Module):
             raise RuntimeError(f"stft: expected a 1D or 2D tensor, but got {x.dim()}D tensor")
         if torch.is_grad_enabled() and x.requires_grad:
             raise NotImplementedError("nnaudio_b200: CFP is forward-only; run under torch.no_grad()")
-        x = _C._dev_f32(x, "x")
+        _C._dev_wave(x, "x")  # fp32, bf16 or fp16; the transform itself runs in fp32
         tfr0 = self._stft_magnitude(x)                       # (B, H, T)
         if drop_edge_frames:
             tfr0 = tfr0[:, :, 1:-1].contiguous()             # cfp.py:151-153

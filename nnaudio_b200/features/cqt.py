@@ -449,7 +449,7 @@ class _DecimateFn(torch.autograd.Function):
     def forward(ctx, sig, fir_row, zero_row, poly, n):
         taps = fir_row.shape[1]
         half = (taps - 1) // 2
-        ctx.n, ctx.half, ctx.L, ctx.poly = n, half, sig.shape[-1], poly
+        ctx.n, ctx.half, ctx.L, ctx.poly, ctx.dtype = n, half, sig.shape[-1], poly, sig.dtype
         padded = torch.nn.functional.pad(sig, (half, half))
         c = _C.cqt1992v2_forward(padded, fir_row, zero_row, None, None, None, n, False,
                                  _C.PAD_CONSTANT, None, 1.0, _C.FMT_COMPLEX, 0.0)
@@ -471,7 +471,7 @@ class _DecimateFn(torch.autograd.Function):
                                  None, 1, False, _C.PAD_CONSTANT, None, 1.0, _C.FMT_COMPLEX, 0.0,
                                  path="tcgen05" if use_tc else "simt")
         d_padded = c[..., 0].permute(0, 2, 1).reshape(g.shape[0], M * n)   # [n*m + p] = phase p, m
-        return d_padded[:, half:half + L].contiguous(), None, None, None, None
+        return d_padded[:, half:half + L].to(ctx.dtype).contiguous(), None, None, None, None
 
 
 class _FirDecimateFn(torch.autograd.Function):
@@ -528,7 +528,10 @@ def _decimate_autograd(mod, tag, sig, fir, n):
 
 def _pyramid_forward_autograd(mod, x, output_format, fallbacks, factor, scale, scale_all, eps):
     """cqt.py:1085-1139 / vqt.py:160-215 octave by octave with autograd-visible stages
-    (training path; inference uses the single fused C call above)."""
+    (training path; inference uses the single fused C call above).  A bf16 / fp16 input enters as
+    its exact fp32 copy (the decimator stages are fp32); autograd casts its gradient back to x.dtype."""
+    if x.dtype in (torch.bfloat16, torch.float16):
+        x = x.float()
     if factor > 1:
         x = _decimate_autograd(mod, "early", x, mod.early_downsample_filter, factor)
     hop = mod.hop_length

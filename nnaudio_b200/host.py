@@ -88,6 +88,9 @@ def alloc_pinned(shape, dtype=torch.float32, device_index: int = 0, fill: Option
     return t, (f"gpu-local node ({len(cpus)} cpus)" if (cpus and old is not None) else "default policy")
 
 
+_X_DTYPES = (torch.float32, torch.bfloat16, torch.float16)
+
+
 class HostPipeline:
     def __init__(self, module: torch.nn.Module, chunk_clips: int = 8, copy_streams: int = 1,
                  **forward_kwargs):
@@ -105,32 +108,34 @@ class HostPipeline:
 
     N_BUF = 3  # input staging buffers: copy-in of chunk c+2 may start while chunk c is transformed
 
-    def _setup(self, device, L):
-        if self._dev != (device, L):
-            self._in = [torch.empty((self.chunk, L), dtype=torch.float32, device=device)
+    def _setup(self, device, L, dtype):
+        if self._dev != (device, L, dtype):
+            self._in = [torch.empty((self.chunk, L), dtype=dtype, device=device)
                         for _ in range(self.N_BUF)]
             self._streams = (torch.cuda.Stream(device), torch.cuda.Stream(device))
             self._extra_in = [torch.cuda.Stream(device) for _ in range(self.n_in - 1)]
             self._done_compute = [None] * self.N_BUF
             self._count = 0
-            self._dev = (device, L)
+            self._dev = (device, L, dtype)
 
     @torch.no_grad()
     def __call__(self, x_host: torch.Tensor, out_host: Optional[torch.Tensor] = None,
                  device: Optional[torch.device] = None) -> torch.Tensor:
-        """x_host: (B, L) fp32 pinned CPU tensor -> spectrograms in a pinned CPU
-        tensor (allocated on first use if ``out_host`` is None).  Asynchronous with
+        """x_host: (B, L) pinned CPU tensor, float32, bfloat16 or float16 -> fp32 spectrograms in a
+        pinned CPU tensor (allocated on first use if ``out_host`` is None).  16-bit audio is copied
+        and transformed as is (half the bytes over the link of fp32); the result equals the
+        module's on the fp32 copy of the same samples.  Asynchronous with
         respect to the host: the CURRENT stream waits for the last copy, so
         ``torch.cuda.current_stream().synchronize()`` (or an event recorded on it)
         marks completion.  ``x_host`` must hold its data when the call is made (it is read
         by the copy engine without waiting for work queued on the current stream)."""
-        if x_host.is_cuda or x_host.dtype != torch.float32 or x_host.dim() != 2:
-            raise ValueError("x_host must be a (B, L) float32 CPU tensor")
+        if x_host.is_cuda or x_host.dtype not in _X_DTYPES or x_host.dim() != 2:
+            raise ValueError("x_host must be a (B, L) float32, bfloat16 or float16 CPU tensor")
         if not x_host.is_pinned():
             raise ValueError("x_host must be pinned (torch.Tensor.pin_memory()) for asynchronous copies")
         device = device or next(self.module.buffers()).device
         B, L = x_host.shape
-        self._setup(device, L)
+        self._setup(device, L, x_host.dtype)
         s_in, s_out = self._streams
         cur = torch.cuda.current_stream(device)
         in_streams = [s_in] + self._extra_in
